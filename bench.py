@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the CPU oracle on the host cores
+    python bench.py ... --dump-outputs DIR                   # also the last timed step's result as DIR/*.npy
 
 One step = one pass of the hot path over one batch of synthetic templated-wiki text (seed 42,
 generated on the device): at N = 1 BASELINE.json configs[1] (10 GB on one B200); at N > 1 every
@@ -51,7 +52,14 @@ def parse_args():
     ap.add_argument("--verify-gib", type=float, default=0.0,
                     help="bytes per rank the CPU oracle re-walks in `verify` (GiB from the shard's entry; 0 = the whole shard)")
     ap.add_argument("--no-oracle", action="store_true", help="skip the CPU-oracle leg of `verify` (cuts, digests, canon)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the result of this project's path (--impl ours)")
+    return args
 
 
 def measured_peak():
@@ -100,6 +108,71 @@ class ClockSampler:
         sm.sort()
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": mx or None, "reasons": sorted(reasons),
                 "samples": len(sm)}
+
+
+DUMP_SEED = 20260   # the rows a dump keeps depend on this seed, the array's length and the number of ranks only
+
+
+def dump_rows(n, cap):
+    """Indices of the rows of an n-row array that a dump keeps: all of them, or a sorted seeded sample of `cap`."""
+    import numpy as np
+    if n <= cap:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, cap, replace=False))
+
+
+def dump_outputs(out_dir, arrays, counts, rank, world):
+    """Writes what the timed path returned in its last step, so that two builds run with the same arguments (the same
+    seeded input) can be compared output for output: DIR/<name>.npy per array and DIR/counts.npy, with the suffix
+    .rank<r> at N > 1.  arrays: name -> (tensor, kind, rows).  kind says how values become float32 / float64 exactly:
+    "byte" (uint8 / bool -> float32), "int" (integers below 2^53 -> float64), "u32" (32-bit patterns -> float64), "u64"
+    (64-bit patterns -> float64 pairs (high, low 32 bits) in a last axis of 2).  rows: the most rows of the array the
+    whole dump keeps, split evenly among the ranks; a rank with more keeps the seeded sample dump_rows(n, rows // N).
+    The callers' row limits keep a dump under 64 MB whatever N is."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    sfx = "" if world == 1 else ".rank%d" % rank
+    for name, (t, kind, rows) in arrays.items():
+        keep = torch.from_numpy(dump_rows(int(t.shape[0]), max(1, rows // world)))
+        a = t[keep.to(t.device)].cpu().numpy()
+        if kind == "byte":
+            a = a.astype(np.float32)
+        elif kind == "u32":
+            a = a.view(np.uint32).astype(np.float64)
+        elif kind == "u64":
+            u = a.view(np.uint64)
+            a = np.stack([u >> np.uint64(32), u & np.uint64(0xFFFFFFFF)], axis=-1).astype(np.float64)
+        else:
+            a = a.astype(np.float64)
+        np.save(os.path.join(out_dir, name + sfx + ".npy"), a)
+    np.save(os.path.join(out_dir, "counts" + sfx + ".npy"), np.array(counts, dtype=np.float64))
+
+
+def dump_ingest(out_dir, res, rank, world):
+    """The IngestResult of --config 2 / 4: cuts, digests [n, 32], canon, is_first, select, offsets, blob and counts =
+    [entry, id_base, chunks, streams, blob bytes].  At most 2^17 rows of each per-chunk / per-stream array and 2^20 bytes
+    of the blob: 26 MB in all."""
+    rows = 1 << 17
+    dump_outputs(out_dir, {"cuts": (res.cuts, "int", rows), "digests": (res.digests, "byte", rows),
+                           "canon": (res.canon, "int", rows), "is_first": (res.is_first, "byte", rows),
+                           "select": (res.select, "int", rows), "offsets": (res.offsets, "int", rows),
+                           "blob": (res.blob, "byte", 1 << 20)},
+                 [res.entry, res.id_base, res.n_chunks, res.select.numel(), res.blob.numel()], rank, world)
+
+
+def dump_similarity(out_dir, out, rank, world):
+    """One step of --config 5: cuts, sig [n, 128], keys [n, 32] (band keys of this rank's chunks), the sorted triples
+    (band, key, id) of the bands this rank owns, and counts = [entry, id_base, chunks of the stream, chunks, triples].
+    At most 2^14 rows of cuts / sig / keys and 2^17 triples: 30 MB in all."""
+    import torch
+    rows, trip = 1 << 14, 1 << 17
+    none = torch.empty(0, dtype=torch.int64)
+    band, key, ids = (none, none, none) if out["band"] is None else (out["band"], out["key"], out["ids"])
+    dump_outputs(out_dir, {"cuts": (out["cuts"], "int", rows), "sig": (out["sig"], "u32", rows),
+                           "keys": (out["keys"], "u64", rows), "band": (band, "int", trip), "key": (key, "u64", trip),
+                           "ids": (ids, "int", trip)},
+                 [out["entry"], out["id_base"], out["n_total"], out["cuts"].numel(), band.numel()], rank, world)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -370,6 +443,8 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     stage_ms = {k: v / args.steps for k, v in stage_ms.items()}
     value = total / (ms * 1e-3) / 1e9
+    if args.dump_outputs:
+        dump_ingest(args.dump_outputs, res, rank, world)
 
     # ---- pipeline facts for the roofline ---------------------------------------------------------
     n_chunks = res.n_chunks
@@ -862,6 +937,8 @@ def run_config4(args):
     clocks = sampler.stop() if rank == 0 else None
     lib.hmse_timing(ctx.h, 0)
     stage_ms = {k: v / args.steps for k, v in stage_ms.items()}
+    if args.dump_outputs:
+        dump_ingest(args.dump_outputs, res, rank, world)
     n_chunks = res.n_chunks
     starts = torch.cat([torch.full((1,), int(res.entry), dtype=torch.int64, device=dev), res.cuts[:-1]])
     lens = res.cuts - starts
@@ -1049,7 +1126,7 @@ def run_config5(args):
                     ids=ids, ev=ev, xs=xs)
 
     out = None
-    for _ in range(max(1, args.warmup)):
+    for _ in range(args.warmup):
         out = None
         torch.cuda.empty_cache()
         out = step(False)
@@ -1077,6 +1154,8 @@ def run_config5(args):
     clocks = sampler.stop() if rank == 0 else None
     lib.hmse_timing(ctx.h, 0)
     st_ms /= args.steps
+    if args.dump_outputs:
+        dump_similarity(args.dump_outputs, out, rank, world)
     n_local = int(out["cuts"].numel())
     n_total = int(out["n_total"])
     own_bytes = int(out["cuts"][-1]) - int(out["entry"]) if n_local else 0

@@ -139,7 +139,3 @@ def test_c_program_sharded_over_nccl_matches_oracle(corpus8, tmp_path, world):
     assert np.array_equal(np.concatenate(all_canon), wcanon)
     assert sorted(triples) == list(zip(wb.tolist(), wk.tolist(), wi.tolist()))
     (tmp_path / "log.txt").write_text(r.stdout)
-    out_dir = os.path.join(ROOT, "gpurun_out")
-    if os.path.isdir(out_dir):
-        with open(os.path.join(out_dir, "c_abi_sharded_world%d.log" % world), "w") as f:
-            f.write(r.stdout + r.stderr)

@@ -3,7 +3,7 @@ base of config 1, and a stream longer than 4 GiB where a 32-bit offset anywhere 
 would show.  The bytes come from the device generator (bit-identical to oracle/corpus.py: checked here on a prefix and on
 windows, and in tests/test_gpu_corpus_lsh.py), are copied to the host, and the oracle (chunk_c = Algorithm 1 in C,
 hashlib SHA-256, the dict dedup) runs over ALL of them: the cut list, every digest, canon and is_first must be equal.
-Determinism criterion: /root/reference VALIDATION_METHODS.md:190-194."""
+Determinism criterion: VALIDATION_METHODS.md:190-194 of the HMSE spec."""
 import zlib
 
 import numpy as np

@@ -61,26 +61,32 @@ def test_murmur3_and_minhash_against_an_independent_implementation():
     """MurmurHash3_x86_32 is a third-party primitive the spec names (murmur3.h, README.md:2573, 2591) and does not
     vendor.  scikit-learn ships its own C++ copy of Appleby's function (sklearn.utils.murmurhash3_32, written by other
     people): the oracle's hash (random keys of every length 0..40, random seeds) and whole MinHash signatures - NumPy
-    and C restatements - must equal what that implementation gives, so the pin does not rest on twelve vectors alone."""
-    sk = pytest.importorskip("sklearn.utils")
-    rng = np.random.default_rng(2024)
-    for n in range(0, 41):
-        for _ in range(8):
-            key = rng.integers(0, 256, n, dtype=np.uint8).tobytes()
-            seed = int(rng.integers(0, 1 << 32))
-            assert oracle.murmur3_32(key, seed) == sk.murmurhash3_32(key, seed=seed, positive=True)
-    data = corpus.generate(6000)
-    cuts = np.array([1000, 1003, 4096, 6000], dtype=np.uint64)      # a 3-byte chunk among them
+    and C restatements - must equal what that implementation gives, so the pin does not rest on twelve vectors alone.
+    Its answers are stored in tests/golden/murmur3_sklearn.json (tests/golden/make_murmur3_golden.py), so the pin holds
+    without scikit-learn; where it is installed, the stored answers are recomputed with it and must be the same."""
+    with open(os.path.join(HERE, "golden", "murmur3_sklearn.json")) as f:
+        golden = json.load(f)
+    assert len(golden["hashes"]) == 41 * 8
+    for key, seed, want in golden["hashes"]:
+        assert oracle.murmur3_32(bytes.fromhex(key), seed) == want
+    mh = golden["minhash"]
+    data = corpus.generate(mh["cuts"][-1])
+    assert hashlib.sha256(data.tobytes()).hexdigest() == mh["input_sha256"], "corpus generator drifted"
+    cuts = np.array(mh["cuts"], dtype=np.uint64)      # a 3-byte chunk among them
     sig = oracle.minhash(data, cuts)
     assert np.array_equal(sig, oracle.minhash_c(data, cuts))
-    raw = data.tobytes()
-    lo = 0
-    for j, hi in enumerate(int(c) for c in cuts):
-        shingles = {raw[i:i + 4] for i in range(lo, hi - 3)}
-        for p in (0, 17, 127):
-            want = min((sk.murmurhash3_32(s, seed=p + 1, positive=True) for s in shingles), default=0xFFFFFFFF)
-            assert int(sig[j, p]) == want
-        lo = hi
+    assert len(mh["mins"]) == cuts.size * 3
+    for j, p, want in mh["mins"]:
+        assert int(sig[j, p]) == want
+    try:
+        import sklearn.utils  # noqa: F401
+    except ImportError:
+        return
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("make_murmur3_golden", os.path.join(HERE, "golden", "make_murmur3_golden.py"))
+    gen = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(gen)
+    assert gen.vectors() == golden
 
 
 def test_zlib_preset_dictionary_framing():
