@@ -1,6 +1,7 @@
-"""GPU DEFLATE vs the CPU model (tests/model, mode 2 = run heads, unconditional skip): per-chunk stream sizes
-must agree exactly on text (same candidate sets, same parse, same Huffman code).  TEST INFRASTRUCTURE."""
-import ctypes as C
+"""GPU DEFLATE vs the CPU model (tests/model, the kernel's parameters): every stream of `python tools/check_model.py
+[MiB]` MiB of corpus text, CDC-chunked with the text dictionary, must equal the model's byte for byte (same candidate
+sets, same parse, same Huffman codes).  Prints the first differences in stream terms.  TEST INFRASTRUCTURE;
+tests/test_gpu_deflate_exact.py runs the same comparison on many more inputs."""
 import os
 import sys
 
@@ -9,37 +10,29 @@ import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import hmse_b200  # noqa: E402
 from oracle import corpus  # noqa: E402
-from tests.model.build import Params, build  # noqa: E402
+from tests.model import exact  # noqa: E402
+from tests.model.inflate_tokens import first_difference  # noqa: E402
 
 
 def main():
     mib = int(sys.argv[1]) if len(sys.argv) > 1 else 4
-    lib = build()
     data = corpus.generate(mib << 20)
     zd = corpus.zdict()
     ctx = hmse_b200.default_context(0)
     cuts = hmse_b200.chunk(data, hmse_b200.CDCConfig(), ctx=ctx)
     blob, offs = hmse_b200.compress(data, cuts, None, zd, ctx=ctx)
-    sizes = np.diff(np.asarray(offs).astype(np.int64))
-    zdn = np.frombuffer(zd, dtype=np.uint8)
-    out = np.zeros(70000, dtype=np.uint8)
-    # own-chunk candidates follow the size class of parse_kernel (OWN_SMALL / OWN_MEDIUM / OWN_LARGE in csrc/deflate.cu)
-    prs = {own: Params(hash_bytes=4, chain_own=own, chain_dict=4, lazy=1, too_far=0, dict_hash_bits=15, mode=2, min_len=0)
-           for own in (2, 3, 4)}
-    st = (C.c_uint32 * 8)()
-    starts = np.concatenate([[0], np.asarray(cuts)[:-1]]).astype(np.int64)
+    offs = np.asarray(offs).astype(np.int64)
+    case = exact.Case("corpus", data, cuts, zd)
+    want = case.expected(exact.Model())
     bad = 0
-    tot_g = tot_m = 0
-    for k, (s, e) in enumerate(zip(starts.tolist(), np.asarray(cuts).astype(np.int64).tolist())):
-        ch = np.ascontiguousarray(data[s:e])
-        pr = prs[2 if e - s <= 13312 else 3 if e - s <= 20480 else 4]
-        r = lib.model_compress(ch.ctypes.data, e - s, zdn.ctypes.data, len(zd), C.byref(pr), out.ctypes.data, out.size, st)
-        tot_g += int(sizes[k]); tot_m += int(r)
-        if r != sizes[k]:
+    for k, w in enumerate(want):
+        g = blob[offs[k]:offs[k + 1]].tobytes()
+        if g != w:
             bad += 1
             if bad <= 5:
-                print("chunk", k, "len", e - s, "gpu", int(sizes[k]), "model", int(r))
-    print("chunks", len(starts), "mismatching sizes", bad, "gpu total", tot_g, "model total", tot_m)
+                n = len(case.chunk(k))
+                print("chunk", k, "len", n, exact.size_class(n), "gpu", len(g), "model", len(w), "-", first_difference(g, w))
+    print("chunks", len(want), "differing streams", bad, "gpu bytes", int(offs[-1]), "model bytes", sum(len(w) for w in want))
 
 
 if __name__ == "__main__":
