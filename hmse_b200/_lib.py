@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libhmse_b200.so")
 
 HMSE_OK, HMSE_E_INVAL, HMSE_E_CAPACITY, HMSE_E_CUDA, HMSE_E_NOMEM, HMSE_E_NCCL = 0, -1, -2, -3, -4, -5
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 
 class HmseError(RuntimeError):
@@ -41,6 +41,7 @@ SIGNATURES = {
     "hmse_scratch_bytes": (_U64, [_P]),
     "hmse_guard_check": (_I, [_P]),
     "hmse_chunk": (_I, [_P, _P, _U64, C.POINTER(CdcCfg), _P, _U64, _PU64, _P]),
+    "hmse_chunk_files": (_I, [_P, _P, _U64, _P, _U64, C.POINTER(CdcCfg), _P, _U64, _PU64, _P, _P]),
     "hmse_chunk_scan": (_I, [_P, _P, _U64, C.POINTER(CdcCfg), _P]),
     "hmse_chunk_resolve": (_I, [_P, _P, _U64, _U64, _I, _U64, _P, _U64, _PU64, _PU64, _P]),
     "hmse_chunk_candidates": (_I, [_P, _P, _P, _U64, _P]),

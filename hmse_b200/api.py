@@ -123,6 +123,20 @@ class Context:
                                        C.byref(nc), self.stream))
         return cuts[:nc.value]
 
+    def chunk_files(self, d: torch.Tensor, file_off: torch.Tensor, cfg: CDCConfig):
+        """(cuts int64, file_chunk int64[F+1]): file f = d[file_off[f]:file_off[f+1]] chunked on its own (hmse_chunk_files);
+        file_off is an int64 device tensor of F+1 offsets from 0 to d.numel()."""
+        n, nf = d.numel(), file_off.numel() - 1
+        if nf < 0:
+            raise ValueError("file_off needs at least one entry")
+        cap = n // cfg.min_size + nf + 1
+        cuts = self.empty(cap, torch.int64)
+        fc = self.empty(nf + 1, torch.int64)
+        nc = C.c_uint64(0)
+        self.check(self.lib.hmse_chunk_files(self.h, d.data_ptr(), n, file_off.data_ptr(), nf, C.byref(self.cdc_struct(cfg)),
+                                             cuts.data_ptr(), cap, C.byref(nc), fc.data_ptr(), self.stream))
+        return cuts[:nc.value], fc
+
     def chunk_scan(self, d: torch.Tensor, cfg: CDCConfig):
         self.check(self.lib.hmse_chunk_scan(self.h, d.data_ptr(), d.numel(), C.byref(self.cdc_struct(cfg)), self.stream))
 
@@ -410,6 +424,32 @@ def chunk(data, cfg: CDCConfig = CDCConfig(), ctx: Optional[Context] = None):
     ctx = ctx or default_context()
     cuts = ctx.chunk(ctx.stage(data), cfg)
     return cuts if _is_dev(data) else _np_u64(cuts)
+
+
+def file_offsets(sizes, n: int, ctx: Context) -> torch.Tensor:
+    """int64 device tensor [F+1]: 0, then the running sum of the file sizes (which must add up to n)."""
+    if _is_dev(sizes):
+        sz = sizes.to(torch.int64)
+        off = torch.cat([torch.zeros(1, dtype=torch.int64, device=sz.device), torch.cumsum(sz, 0)])
+        return off.to(ctx.tdev)
+    sz = np.asarray(sizes, dtype=np.int64).reshape(-1)
+    if (sz < 0).any():
+        raise ValueError("file sizes must be >= 0")
+    off = np.concatenate([[0], np.cumsum(sz)]).astype(np.int64)
+    if int(off[-1]) != n:
+        raise ValueError("file sizes add up to %d, the data has %d bytes" % (int(off[-1]), n))
+    return torch.from_numpy(off).to(ctx.tdev)
+
+
+def chunk_files(data, sizes, cfg: CDCConfig = CDCConfig(), ctx: Optional[Context] = None):
+    """Many files in one call: `data` holds the files back to back, `sizes[f]` bytes each (0 allowed).  Every file is
+    chunked on its own, exactly as chunk() chunks it alone.  Returns (cuts uint64[n], file_chunk uint64[F+1]): one chunk
+    list over the whole buffer (absolute offsets), and the index of each file's first chunk (an empty file shares the
+    index of the next file; file_chunk[F] = n).  Host input gives numpy arrays, CUDA input CUDA tensors."""
+    ctx = ctx or default_context()
+    d = ctx.stage(data)
+    cuts, fc = ctx.chunk_files(d, file_offsets(sizes, d.numel(), ctx), cfg)
+    return (cuts, fc) if _is_dev(data) else (_np_u64(cuts), _np_u64(fc))
 
 
 def digest(data, cuts, start0: int = 0, ctx: Optional[Context] = None):

@@ -450,6 +450,25 @@ TmapEncodeFn tmap_encoder() {
 // ------------------------------------------------------------------------------------------
 // K2: resolve
 // ------------------------------------------------------------------------------------------
+// The resolve walks a table of segments.  A segment owns the chunk starts in [start, end) and never cuts past file_end.
+// A head segment knows its entry (segment 0: ResolveArgs::entry, any other head: its start, the first byte of a file);
+// every other segment speculates from its start and is fixed up from its predecessor's exit.  The single stream
+// (hmse_chunk_resolve) is one file whose only head is segment 0; hmse_chunk_files makes one head per non-empty file.
+// A cut decision for a chunk starting at s reads no byte before s (the bitmaps only from s + min_size + 64 on, and a bit
+// depends on the 64 bytes ending at its position), so one scan of the whole buffer serves every file in it.
+struct SegDesc {
+    uint64_t start;     // cuts are stored relative to it
+    uint64_t end;       // chunk starts >= end belong to the next segment
+    uint64_t file_end;  // end of the bytes the chain may use (file end, or the available bytes of a shard)
+    uint64_t list;      // first entry of its spec / pre lists
+    uint32_t cap;       // entries of each list
+    uint32_t head;
+};
+// Starts in [start, end) lie at least min_size apart, so a segment holds at most end/mn - start/mn + 1 of them.  A file
+// table gives segment k cap = end/mn - start/mn + 2 entries at list = start/mn + 2 k (consecutive lists never overlap,
+// the total is n/mn + 2 n_seg: scratch follows the bytes, not the file count); the implicit table of one stream gives
+// every segment seg_len/mn + 2 entries at k (seg_len/mn + 2).
+
 struct SegMeta {
     uint64_t spec_entry;  // start the speculative chain was walked from
     uint64_t cur_entry;   // start the current (pre + spec tail) list is valid for
@@ -463,13 +482,13 @@ struct ResolveArgs {
     const uint64_t* bitS;
     const uint64_t* bitL;
     const CdcDev* cfg;
-    uint64_t n;       // bytes available (clamps at eof)
-    uint64_t n_own;   // starts >= n_own belong to the next shard
-    uint64_t seg_len, n_seg, seg_cap;
-    uint32_t* spec;   // [n_seg][seg_cap] cuts relative to seg_start
-    uint32_t* pre;    // [n_seg][seg_cap]
+    const SegDesc* seg;   // the file table (kernels <true>); the <false> kernels use the implicit table of one stream
+    uint64_t n_seg;
+    uint64_t seg_len, n_own, n_avail, stride;   // (the implicit table)
+    uint32_t* spec;   // speculative cut lists, relative to the segment start, at seg[k].list
+    uint32_t* pre;    // fix-up cut lists, same layout
     SegMeta* meta;
-    uint64_t entry;
+    uint64_t entry;   // where the chain of segment 0 starts
 };
 
 __device__ __forceinline__ uint64_t find_first(const uint64_t* __restrict__ bits, uint64_t lo, uint64_t hi,
@@ -493,12 +512,12 @@ __device__ __forceinline__ uint64_t find_first(const uint64_t* __restrict__ bits
     return ~0ull;
 }
 
-// One application of FastCDC Algorithm 1 to the chunk starting at s (warp-cooperative,
+// One application of FastCDC Algorithm 1 to the chunk starting at s of a stream that ends at fe (warp-cooperative,
 // all lanes return the same value).  sg = gear table in shared memory.
 __device__ __forceinline__ uint64_t next_cut_warp(const ResolveArgs& a, const uint64_t* sg, uint64_t ms, uint64_t ml,
-                                                  uint32_t mn, uint32_t av, uint32_t mx, uint64_t s, unsigned lane) {
-    const uint64_t rem = a.n - s;
-    if (rem <= mn) return a.n;
+                                                  uint32_t mn, uint32_t av, uint32_t mx, uint64_t fe, uint64_t s, unsigned lane) {
+    const uint64_t rem = fe - s;
+    if (rem <= mn) return fe;
     const uint64_t end = s + (rem < mx ? rem : (uint64_t)mx);
     const uint64_t normal = s + ((end - s) < av ? (end - s) : (uint64_t)av);
     const uint64_t base = s + mn;
@@ -539,29 +558,45 @@ __device__ __forceinline__ uint64_t next_cut_warp(const ResolveArgs& a, const ui
 
 constexpr int K2_THREADS = 128;
 
+// Segment k.  TABLE: the file table.  Otherwise the implicit table of one stream, from the kernel parameters (no table
+// load, no registers for the bounds): segments of seg_len bytes over [0, n_own), every chain may read up to n_avail,
+// segment 0 is the only head.
+template <bool TABLE>
+__device__ __forceinline__ SegDesc seg_at(const ResolveArgs& a, uint64_t k) {
+    if constexpr (TABLE) return a.seg[k];
+    SegDesc g;
+    g.start = k * a.seg_len;
+    g.end = g.start + a.seg_len < a.n_own ? g.start + a.seg_len : a.n_own;
+    g.file_end = a.n_avail;
+    g.list = k * a.stride;
+    g.cap = (uint32_t)a.stride;
+    g.head = k == 0;
+    return g;
+}
+
 __device__ __forceinline__ void load_gear(uint64_t* sg, const CdcDev* cfg) {
     for (int i = threadIdx.x; i < 256; i += blockDim.x) sg[i] = cfg->gear[i];
     __syncthreads();
 }
 
+template <bool TABLE>
 __global__ void __launch_bounds__(K2_THREADS) resolve_spec_kernel(ResolveArgs a) {
     __shared__ uint64_t sg[256];
     load_gear(sg, a.cfg);
     const unsigned lane = threadIdx.x & 31;
     const uint64_t k = (uint64_t)blockIdx.x * (K2_THREADS / 32) + (threadIdx.x >> 5);
     if (k >= a.n_seg) return;
+    const SegDesc g = seg_at<TABLE>(a, k);
+    uint64_t s = k == 0 ? a.entry : g.start;
     const uint64_t ms = a.cfg->ms, ml = a.cfg->ml;
     const uint32_t mn = a.cfg->mn, av = a.cfg->av, mx = a.cfg->mx;
-    const uint64_t seg_start = k * a.seg_len;
-    uint64_t seg_end = seg_start + a.seg_len;
-    if (seg_end > a.n_own) seg_end = a.n_own;
-    uint32_t* spec = a.spec + k * a.seg_cap;
-    uint64_t s = k == 0 ? a.entry : seg_start;
+    const uint32_t cap = g.cap;
+    uint32_t* spec = a.spec + g.list;
     const uint64_t s0 = s;
     uint32_t cnt = 0;
-    while (s < seg_end) {
-        uint64_t c = next_cut_warp(a, sg, ms, ml, mn, av, mx, s, lane);
-        if (lane == 0 && cnt < a.seg_cap) spec[cnt] = (uint32_t)(c - seg_start);
+    while (s < g.end) {
+        uint64_t c = next_cut_warp(a, sg, ms, ml, mn, av, mx, g.file_end, s, lane);
+        if (lane == 0 && cnt < cap) spec[cnt] = (uint32_t)(c - g.start);
         cnt++;
         s = c;
     }
@@ -580,8 +615,9 @@ __global__ void __launch_bounds__(K2_THREADS) resolve_spec_kernel(ResolveArgs a)
     }
 }
 
-// One fix-up round: segment k re-enters at exit[in][k-1] (segment 0 at a.entry) and walks until
-// its chain merges with the speculative chain or leaves the segment.
+// One fix-up round: a continuation segment re-enters at its predecessor's exit[in] (a head at its own entry) and walks
+// until its chain merges with the speculative chain or leaves the segment.
+template <bool TABLE>
 __global__ void __launch_bounds__(K2_THREADS) resolve_fix_kernel(ResolveArgs a, int in, uint32_t* changed) {
     __shared__ uint64_t sg[256];
     load_gear(sg, a.cfg);
@@ -590,7 +626,8 @@ __global__ void __launch_bounds__(K2_THREADS) resolve_fix_kernel(ResolveArgs a, 
     if (k >= a.n_seg) return;
     const int out = in ^ 1;
     SegMeta* m = a.meta + k;
-    const uint64_t e = k == 0 ? a.entry : a.meta[k - 1].exit[in];
+    const SegDesc g = seg_at<TABLE>(a, k);
+    const uint64_t e = g.head ? (k == 0 ? a.entry : g.start) : a.meta[k - 1].exit[in];
     const uint64_t old_exit = m->exit[in];
     if (e == m->cur_entry) {
         if (lane == 0) m->exit[out] = old_exit;
@@ -598,11 +635,9 @@ __global__ void __launch_bounds__(K2_THREADS) resolve_fix_kernel(ResolveArgs a, 
     }
     const uint64_t ms = a.cfg->ms, ml = a.cfg->ml;
     const uint32_t mn = a.cfg->mn, av = a.cfg->av, mx = a.cfg->mx;
-    const uint64_t seg_start = k * a.seg_len;
-    uint64_t seg_end = seg_start + a.seg_len;
-    if (seg_end > a.n_own) seg_end = a.n_own;
-    const uint32_t* spec = a.spec + k * a.seg_cap;
-    uint32_t* pre = a.pre + k * a.seg_cap;
+    const uint32_t cap = g.cap;
+    const uint32_t* spec = a.spec + g.list;
+    uint32_t* pre = a.pre + g.list;
     const uint64_t spec_entry = m->spec_entry;
     const uint32_t spec_cnt = m->spec_cnt;
     uint64_t s = e;
@@ -610,9 +645,9 @@ __global__ void __launch_bounds__(K2_THREADS) resolve_fix_kernel(ResolveArgs a, 
     bool merged = false;
     // chunk starts on the speculative chain: start(0) = spec_entry, start(i) = seg_start + spec[i-1]
     uint64_t sstart = spec_entry;
-    while (s < seg_end) {
+    while (s < g.end) {
         while (si < spec_cnt && sstart < s) {
-            sstart = seg_start + spec[si];
+            sstart = g.start + spec[si];
             si++;
         }
         // si == number of spec cuts consumed; sstart is start(si) when si < spec_cnt or the spec exit
@@ -620,8 +655,8 @@ __global__ void __launch_bounds__(K2_THREADS) resolve_fix_kernel(ResolveArgs a, 
             merged = true;
             break;
         }
-        uint64_t c = next_cut_warp(a, sg, ms, ml, mn, av, mx, s, lane);
-        if (lane == 0 && pc < a.seg_cap) pre[pc] = (uint32_t)(c - seg_start);
+        uint64_t c = next_cut_warp(a, sg, ms, ml, mn, av, mx, g.file_end, s, lane);
+        if (lane == 0 && pc < cap) pre[pc] = (uint32_t)(c - g.start);
         pc++;
         s = c;
     }
@@ -641,21 +676,163 @@ __global__ void seg_counts_kernel(const SegMeta* __restrict__ meta, uint64_t n_s
     if (k < n_seg) counts[k] = (uint64_t)meta[k].pre_cnt + meta[k].spec_cnt - meta[k].spec_skip;
 }
 
+template <bool TABLE>
 __global__ void __launch_bounds__(K2_THREADS)
 seg_gather_kernel(ResolveArgs a, const uint64_t* __restrict__ offs, uint64_t cap, uint64_t* __restrict__ cuts) {
     const unsigned lane = threadIdx.x & 31;
     const uint64_t k = (uint64_t)blockIdx.x * (K2_THREADS / 32) + (threadIdx.x >> 5);
     if (k >= a.n_seg) return;
     const SegMeta m = a.meta[k];
-    const uint64_t seg_start = k * a.seg_len;
-    const uint32_t* spec = a.spec + k * a.seg_cap;
-    const uint32_t* pre = a.pre + k * a.seg_cap;
+    const SegDesc g = seg_at<TABLE>(a, k);
+    const uint64_t seg_start = g.start, list = g.list;
+    const uint32_t* spec = a.spec + list;
+    const uint32_t* pre = a.pre + list;
     const uint64_t o = offs[k];
     const uint32_t cnt = m.pre_cnt + m.spec_cnt - m.spec_skip;
     for (uint32_t i = lane; i < cnt; i += 32) {
         uint32_t rel = i < m.pre_cnt ? pre[i] : spec[m.spec_skip + (i - m.pre_cnt)];
         if (o + i < cap) cuts[o + i] = seg_start + rel;
     }
+}
+
+// File table, step 1 (one thread per offset i <= n_files): off[0] == 0, off never decreases, off[n_files] == n; nseg[f] =
+// segments of file f (0 for an empty file, and for any file whose offsets are bad: *bad is then set).
+__global__ void file_count_kernel(const uint64_t* __restrict__ off, uint64_t n_files, uint64_t n, uint64_t seg_len,
+                                  uint64_t* __restrict__ nseg, uint32_t* __restrict__ bad) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i > n_files) return;
+    const uint64_t hi = off[i];
+    const uint64_t lo = i ? off[i - 1] : 0;
+    const bool ok = hi <= n && lo <= hi && (i || hi == 0) && (i < n_files || hi == n);
+    if (!ok) atomicOr(bad, 1u);
+    if (i) nseg[i - 1] = ok ? (hi - lo + seg_len - 1) / seg_len : 0;
+}
+
+// File table, step 2 (one thread per segment): first[f] = index of file f's first segment (exclusive scan of nseg), so
+// segment k belongs to the last file f with first[f] <= k (files before it with the same first[] are empty).
+__global__ void file_table_kernel(const uint64_t* __restrict__ off, const uint64_t* __restrict__ first, uint64_t n_files,
+                                  uint64_t n_seg, uint64_t seg_len, uint32_t mn, SegDesc* __restrict__ seg) {
+    const uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n_seg) return;
+    uint64_t lo = 0, hi = n_files - 1;   // invariant: first[lo] <= k (first[0] == 0), answer in [lo, hi]
+    while (lo < hi) {
+        const uint64_t mid = lo + (hi - lo + 1) / 2;
+        if (__ldg(first + mid) <= k) lo = mid;
+        else hi = mid - 1;
+    }
+    const uint64_t j = k - first[lo];
+    const uint64_t fe = off[lo + 1];
+    SegDesc g;
+    g.start = off[lo] + j * seg_len;
+    g.end = g.start + seg_len < fe ? g.start + seg_len : fe;
+    g.file_end = fe;
+    g.list = g.start / mn + 2 * k;
+    g.cap = (uint32_t)(g.end / mn - g.start / mn + 2);
+    g.head = j == 0;
+    seg[k] = g;
+}
+
+// file_chunk[f] = index of file f's first chunk = chunk offset of its head segment; an empty file shares the index of
+// the next non-empty one (or the total); file_chunk[n_files] = total.
+__global__ void file_chunk_kernel(const uint64_t* __restrict__ first, const uint64_t* __restrict__ offs, uint64_t n_files,
+                                  uint64_t n_seg, const uint64_t* __restrict__ total, uint64_t* __restrict__ file_chunk) {
+    const uint64_t f = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (f > n_files) return;
+    const uint64_t s = f < n_files ? first[f] : n_seg;
+    file_chunk[f] = s < n_seg ? offs[s] : (n_seg ? *total : 0);
+}
+
+// Bytes per resolve segment: a warp walks at most this many bytes before a fix-up round.
+uint64_t resolve_seg_len(const hmse_cdc_cfg& c) {
+    const uint64_t len = 8ull * c.max_size;
+    return len < (256u << 10) ? (256u << 10) : len;
+}
+
+// Scratch of a resolve over n_seg segments whose last one ends at last_end: lists in SLOT_CDC_SEG, and in SLOT_CDC_META
+// [SegMeta n_seg][SegDesc n_seg][counts u64 n_seg][offs u64 n_seg][tail: changed flag u32, total u64, ...].
+struct ResolveScratch {
+    ResolveArgs a;
+    SegDesc* seg;
+    uint64_t *counts, *offs, *tail;
+};
+
+int resolve_scratch(hmse_ctx* ctx, uint64_t n_seg, uint64_t last_end, const uint8_t* d_data, uint64_t n_avail,
+                    uint64_t entry, bool file_table, ResolveScratch* r) {
+    const uint64_t mn = ctx->cdc_cfg.min_size, stride = resolve_seg_len(ctx->cdc_cfg) / mn + 2;
+    const uint64_t list_entries = file_table ? last_end / mn + 2 * n_seg : n_seg * stride;
+    HMSE_SCRATCH(ctx, lists, uint32_t*, SLOT_CDC_SEG, 2 * list_entries * sizeof(uint32_t));
+    const size_t meta_bytes = n_seg * (sizeof(SegMeta) + sizeof(SegDesc)) + 2 * n_seg * sizeof(uint64_t) + 64;
+    HMSE_SCRATCH(ctx, meta_raw, uint8_t*, SLOT_CDC_META, meta_bytes);
+    const uint64_t n_tiles = div_up64(n_avail, K1_TILE);
+    const uint64_t words = (n_tiles ? n_tiles : 1) * (K1_TILE / 64);
+    ResolveArgs& a = r->a;
+    a.data = d_data;
+    a.bitS = (const uint64_t*)ctx->slot[SLOT_CDC_BITS];
+    a.bitL = a.bitS + words;
+    a.cfg = (const CdcDev*)ctx->slot[SLOT_CDC_CFG];
+    a.meta = (SegMeta*)meta_raw;
+    r->seg = (SegDesc*)(meta_raw + n_seg * sizeof(SegMeta));
+    a.seg = file_table ? r->seg : nullptr;
+    a.n_seg = n_seg;
+    a.seg_len = resolve_seg_len(ctx->cdc_cfg);
+    a.n_own = last_end;
+    a.n_avail = n_avail;
+    a.stride = stride;
+    a.spec = lists;
+    a.pre = lists + list_entries;
+    a.entry = entry;
+    r->counts = (uint64_t*)(meta_raw + n_seg * (sizeof(SegMeta) + sizeof(SegDesc)));
+    r->offs = r->counts + n_seg;
+    r->tail = r->offs + n_seg;
+    return HMSE_OK;
+}
+
+// Speculative walk (fresh) or the exits of the previous call, fix-up rounds until no exit changes (one host round trip
+// each), then counts, their scan (total in tail[1]) and the gather into d_cuts[cap].  Leaves the round count and the
+// parity of the final exits in ctx->cdc_rounds; *in_out = that parity.
+int resolve_run(hmse_ctx* ctx, const ResolveScratch& r, bool fresh, uint64_t* d_cuts, uint64_t cap, int* in_out,
+                cudaStream_t st) {
+    const ResolveArgs& a = r.a;
+    const unsigned wgrid = (unsigned)div_up64(a.n_seg, K2_THREADS / 32);
+    int in = 0;
+    int rounds = 0;
+    if (fresh) {
+        KL(ctx);
+        if (a.seg) resolve_spec_kernel<true><<<wgrid, K2_THREADS, 0, st>>>(a);
+        else resolve_spec_kernel<false><<<wgrid, K2_THREADS, 0, st>>>(a);
+        HMSE_LAUNCH_CHECK(ctx);
+    } else {
+        in = ctx->cdc_rounds & 1;  // parity the previous call's final exits live in
+    }
+    volatile uint64_t* mail = ctx->pinned;
+    for (;;) {
+        HMSE_CUDA(ctx, cudaMemsetAsync(r.tail, 0, 8, st));
+        KL(ctx);
+        if (a.seg) resolve_fix_kernel<true><<<wgrid, K2_THREADS, 0, st>>>(a, in, (uint32_t*)r.tail);
+        else resolve_fix_kernel<false><<<wgrid, K2_THREADS, 0, st>>>(a, in, (uint32_t*)r.tail);
+        HMSE_LAUNCH_CHECK(ctx);
+        if (int mrc = hmse_mail(ctx, 0, r.tail, 2, st)) return mrc;
+        HMSE_CUDA(ctx, cudaStreamSynchronize(st));
+        in ^= 1;
+        rounds++;
+        if ((uint32_t)mail[0] == 0) break;
+        if ((uint64_t)rounds > a.n_seg + 2) HMSE_FAIL(ctx, HMSE_E_CUDA, "resolve did not converge");
+    }
+    ctx->cdc_rounds = (rounds << 1) | in;  // low bit: parity the final exits live in
+    *in_out = in;
+
+    KL(ctx);
+    seg_counts_kernel<<<(unsigned)div_up64(a.n_seg, 256), 256, 0, st>>>(a.meta, a.n_seg, r.counts);
+    HMSE_LAUNCH_CHECK(ctx);
+    int rc = hmse_exclusive_scan_u64(ctx, r.counts, r.offs, a.n_seg, r.tail + 1, st);
+    if (rc) return rc;
+    if (d_cuts && cap) {
+        KL(ctx);
+        if (a.seg) seg_gather_kernel<true><<<wgrid, K2_THREADS, 0, st>>>(a, r.offs, cap, d_cuts);
+        else seg_gather_kernel<false><<<wgrid, K2_THREADS, 0, st>>>(a, r.offs, cap, d_cuts);
+        HMSE_LAUNCH_CHECK(ctx);
+    }
+    return HMSE_OK;
 }
 
 int upload_cfg(hmse_ctx* ctx, const hmse_cdc_cfg* cfg, cudaStream_t st) {
@@ -806,89 +983,86 @@ HMSE_API int hmse_chunk_resolve(hmse_ctx* ctx, const uint8_t* d_data, uint64_t n
     if (exit_off) *exit_off = entry;
     if (n_own == 0 || entry >= n_own) return HMSE_OK;
 
-    uint64_t seg_len = 8ull * c.max_size;
-    if (seg_len < (256u << 10)) seg_len = 256u << 10;
+    const uint64_t seg_len = resolve_seg_len(c);
     if (entry >= seg_len) HMSE_FAIL(ctx, HMSE_E_INVAL, "entry must lie in the first segment");
     const uint64_t n_seg = div_up64(n_own, seg_len);
-    const uint64_t seg_cap = seg_len / c.min_size + 2;
-    const uint64_t n_tiles = div_up64(n_avail, K1_TILE);
-    const uint64_t words = (n_tiles ? n_tiles : 1) * (K1_TILE / 64);
-
-    HMSE_SCRATCH(ctx, lists, uint32_t*, SLOT_CDC_SEG, 2 * n_seg * seg_cap * sizeof(uint32_t));
-    // meta: [SegMeta n_seg][counts u64 n_seg][offs u64 n_seg][changed u32, total u64]
-    const size_t meta_bytes = n_seg * sizeof(SegMeta) + 2 * n_seg * sizeof(uint64_t) + 64;
-    HMSE_SCRATCH(ctx, meta_raw, uint8_t*, SLOT_CDC_META, meta_bytes);
-    SegMeta* meta = (SegMeta*)meta_raw;
-    uint64_t* counts = (uint64_t*)(meta_raw + n_seg * sizeof(SegMeta));
-    uint64_t* offs = counts + n_seg;
-    uint64_t* tail = offs + n_seg;  // tail[0] = changed flag (u32), tail[1] = total, tail[2] = exit
-
-    ResolveArgs a;
-    a.data = d_data;
-    a.bitS = (const uint64_t*)ctx->slot[SLOT_CDC_BITS];
-    a.bitL = a.bitS + words;
-    a.cfg = (const CdcDev*)ctx->slot[SLOT_CDC_CFG];
-    a.n = n_avail;
-    a.n_own = n_own;
-    a.seg_len = seg_len;
-    a.n_seg = n_seg;
-    a.seg_cap = seg_cap;
-    a.spec = lists;
-    a.pre = lists + n_seg * seg_cap;
-    a.meta = meta;
-    a.entry = entry;
-
-    const unsigned wgrid = (unsigned)div_up64(n_seg, K2_THREADS / 32);
+    ResolveScratch r;
+    if (int rc = resolve_scratch(ctx, n_seg, n_own, d_data, n_avail, entry, false, &r)) return rc;
+    // the segment records of the previous call are reused when they belong to the same shard geometry (incremental
+    // re-resolve with another entry); hmse_chunk_scan and hmse_chunk_files clear res_valid
     const bool fresh = !(ctx->res_valid && ctx->res_n_own == n_own && ctx->res_eof == eof && ctx->seg_len == seg_len &&
-                         ctx->n_seg == n_seg && ctx->seg_cap == seg_cap);
-    int in = 0;
-    int rounds = 0;
+                         ctx->n_seg == n_seg);
     HT_BEGIN(ctx, HT_RESOLVE, st);
-    if (fresh) {
-        KL(ctx);
-        resolve_spec_kernel<<<wgrid, K2_THREADS, 0, st>>>(a);
-        HMSE_LAUNCH_CHECK(ctx);
-    } else {
-        in = ctx->cdc_rounds & 1;  // parity the previous call's final exits live in
-    }
-    volatile uint64_t* mail = ctx->pinned;
-    for (;;) {
-        HMSE_CUDA(ctx, cudaMemsetAsync(tail, 0, 8, st));
-        KL(ctx);
-        resolve_fix_kernel<<<wgrid, K2_THREADS, 0, st>>>(a, in, (uint32_t*)tail);
-        HMSE_LAUNCH_CHECK(ctx);
-        if (int mrc = hmse_mail(ctx, 0, tail, 2, st)) return mrc;
-        HMSE_CUDA(ctx, cudaStreamSynchronize(st));
-        in ^= 1;
-        rounds++;
-        if ((uint32_t)mail[0] == 0) break;
-        if ((uint64_t)rounds > n_seg + 2) HMSE_FAIL(ctx, HMSE_E_CUDA, "resolve did not converge");
-    }
-    ctx->cdc_rounds = (rounds << 1) | in;  // low bit: parity the final exits live in
+    ctx->res_valid = 0;
+    int in = 0;
+    if (int rc = resolve_run(ctx, r, fresh, d_cuts, cap, &in, st)) return rc;
     ctx->res_valid = 1;
     ctx->res_n_own = n_own;
     ctx->res_eof = eof;
     ctx->seg_len = seg_len;
     ctx->n_seg = n_seg;
-    ctx->seg_cap = seg_cap;
-
-    KL(ctx);
-    seg_counts_kernel<<<(unsigned)div_up64(n_seg, 256), 256, 0, st>>>(meta, n_seg, counts);
-    HMSE_LAUNCH_CHECK(ctx);
-    int rc = hmse_exclusive_scan_u64(ctx, counts, offs, n_seg, tail + 1, st);
-    if (rc) return rc;
-    if (d_cuts && cap) {
-        KL(ctx);
-        seg_gather_kernel<<<wgrid, K2_THREADS, 0, st>>>(a, offs, cap, d_cuts);
-        HMSE_LAUNCH_CHECK(ctx);
-    }
     HT_END(ctx, HT_RESOLVE, st);
-    if (int mrc = hmse_mail(ctx, 0, tail + 1, 2, st)) return mrc;
-    if (int mrc = hmse_mail(ctx, 2, &meta[n_seg - 1].exit[in], 2, st)) return mrc;
+    volatile uint64_t* mail = ctx->pinned;
+    if (int mrc = hmse_mail(ctx, 0, r.tail + 1, 2, st)) return mrc;
+    if (int mrc = hmse_mail(ctx, 2, &r.a.meta[n_seg - 1].exit[in], 2, st)) return mrc;
     HMSE_CUDA(ctx, cudaStreamSynchronize(st));
     *n_cuts = mail[0];
     if (exit_off) *exit_off = mail[1];
     if (!d_cuts || mail[0] > cap)
+        HMSE_FAIL(ctx, HMSE_E_CAPACITY, "d_cuts capacity %llu < %llu cuts", (unsigned long long)cap,
+                  (unsigned long long)mail[0]);
+    return HMSE_OK;
+}
+
+HMSE_API int hmse_chunk_files(hmse_ctx* ctx, const uint8_t* d_data, uint64_t n, const uint64_t* d_file_off, uint64_t n_files,
+                              const hmse_cdc_cfg* cfg, uint64_t* d_cuts, uint64_t cap, uint64_t* n_cuts,
+                              uint64_t* d_file_chunk, void* stream) {
+    if (!ctx) return HMSE_E_INVAL;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!n_cuts || !d_file_off || !d_file_chunk) HMSE_FAIL(ctx, HMSE_E_INVAL, "hmse_chunk_files: null pointer");
+    *n_cuts = 0;
+    if (int rc = hmse_chunk_scan(ctx, d_data, n, cfg, stream)) return rc;   // (clears res_valid)
+    const hmse_cdc_cfg& c = ctx->cdc_cfg;
+    const uint64_t seg_len = resolve_seg_len(c);
+    // [first u64 n_files][bad u32 | n_seg u64 | ...]
+    HMSE_SCRATCH(ctx, files, uint64_t*, SLOT_CDC_FILES, n_files * sizeof(uint64_t) + 64);
+    uint64_t* ftail = files + n_files;
+    volatile uint64_t* mail = ctx->pinned;
+    HT_BEGIN(ctx, HT_RESOLVE, st);
+    HMSE_CUDA(ctx, cudaMemsetAsync(ftail, 0, 16, st));
+    KL(ctx);
+    file_count_kernel<<<(unsigned)div_up64(n_files + 1, 256), 256, 0, st>>>(d_file_off, n_files, n, seg_len, files,
+                                                                            (uint32_t*)ftail);
+    HMSE_LAUNCH_CHECK(ctx);
+    if (int rc = hmse_exclusive_scan_u64(ctx, files, files, n_files, ftail + 1, st)) return rc;
+    if (int mrc = hmse_mail(ctx, 0, ftail, 4, st)) return mrc;
+    HMSE_CUDA(ctx, cudaStreamSynchronize(st));
+    if ((uint32_t)mail[0])
+        HMSE_FAIL(ctx, HMSE_E_INVAL, "hmse_chunk_files: file offsets must start at 0, never decrease and end at n = %llu",
+                  (unsigned long long)n);
+    const uint64_t n_seg = mail[1];
+    ResolveScratch r;
+    if (int rc = resolve_scratch(ctx, n_seg, n, d_data, n, 0, true, &r)) return rc;
+    int in = 0;
+    if (n_seg) {
+        KL(ctx);
+        file_table_kernel<<<(unsigned)div_up64(n_seg, 256), 256, 0, st>>>(d_file_off, files, n_files, n_seg, seg_len,
+                                                                         c.min_size, r.seg);
+        HMSE_LAUNCH_CHECK(ctx);
+        if (int rc = resolve_run(ctx, r, true, d_cuts, cap, &in, st)) return rc;
+    } else {
+        HMSE_CUDA(ctx, cudaMemsetAsync(r.tail + 1, 0, 8, st));
+        ctx->cdc_rounds = 0;
+    }
+    KL(ctx);
+    file_chunk_kernel<<<(unsigned)div_up64(n_files + 1, 256), 256, 0, st>>>(files, r.offs, n_files, n_seg, r.tail + 1,
+                                                                            d_file_chunk);
+    HMSE_LAUNCH_CHECK(ctx);
+    HT_END(ctx, HT_RESOLVE, st);
+    if (int mrc = hmse_mail(ctx, 0, r.tail + 1, 2, st)) return mrc;
+    HMSE_CUDA(ctx, cudaStreamSynchronize(st));
+    *n_cuts = mail[0];
+    if (mail[0] > cap || (mail[0] && !d_cuts))
         HMSE_FAIL(ctx, HMSE_E_CAPACITY, "d_cuts capacity %llu < %llu cuts", (unsigned long long)cap,
                   (unsigned long long)mail[0]);
     return HMSE_OK;

@@ -13,7 +13,8 @@ enum HmseSlot {
     SLOT_CDC_CFG = 0,   // device copy of gear table + parameters (CdcDev)
     SLOT_CDC_BITS,      // MaskS / MaskL candidate bitmaps, one bit per byte each
     SLOT_CDC_SEG,       // per-segment speculative + fix-up cut lists
-    SLOT_CDC_META,      // per-segment entry/exit/count records, flags
+    SLOT_CDC_META,      // per-segment entry/exit/count records and segment table, flags
+    SLOT_CDC_FILES,     // first segment of every file (hmse_chunk_files)
     SLOT_SCAN,          // block sums of the generic exclusive scan
     SLOT_SHA_MISC,      // work counter
     SLOT_DEDUP_TABLE,   // open-addressing table of chunk indices
@@ -69,7 +70,7 @@ struct hmse_ctx {
     int cdc_have_scan;
     int cdc_rounds;
     // resolve state (incremental re-resolve)
-    uint64_t seg_len, n_seg, seg_cap;
+    uint64_t seg_len, n_seg;
     uint64_t res_n_own;
     int res_eof, res_valid;
     // per-launch spans of the dominant kernel (parse_kernel) of the last hmse_compress, and what it moved

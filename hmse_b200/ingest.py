@@ -10,7 +10,7 @@ from typing import Optional
 import torch
 
 from . import sharding
-from .api import Context
+from .api import Context, file_offsets
 from .config import CDCConfig, SimConfig
 
 
@@ -28,6 +28,7 @@ class IngestResult:
     base: Optional[torch.Tensor] = None           # L4: int64 [n] base chunk of every chunk stored as a delta, else -1
     delta_blob: Optional[torch.Tensor] = None     # L4: uint8 packed deltas (chunk order)
     delta_offsets: Optional[torch.Tensor] = None  # L4: int64 [n + 1]
+    file_chunk: Optional[torch.Tensor] = None     # files: int64 [F + 1] index of each file's first chunk (run(files=...))
 
     @property
     def n_chunks(self) -> int:
@@ -67,12 +68,21 @@ class Ingest:
         dblob, doffs = ctx.delta_encode(d, cuts, base, start0=start0)
         return base, dblob, doffs
 
-    def run(self, d: torch.Tensor, compress: bool = True, l4: Optional[SimConfig] = None, min_votes: int = 4) -> IngestResult:
+    def run(self, d: torch.Tensor, compress: bool = True, l4: Optional[SimConfig] = None, min_votes: int = 4,
+            files=None) -> IngestResult:
         """l4: also run the similarity layer; first occurrences that keep a delta are not compressed (`select` lists
-        the chunks of the chunk store only) and `base` / `delta_blob` / `delta_offsets` describe the deltas."""
+        the chunks of the chunk store only) and `base` / `delta_blob` / `delta_offsets` describe the deltas.
+        files: the sizes of the files `d` holds back to back (a sequence or an integer tensor, zeros allowed).  Every
+        file is then chunked on its own (hmse_chunk_files): no chunk spans two files, so equal files give equal chunks
+        wherever they sit, and `file_chunk` records where each file's chunks begin.  Everything after chunking runs
+        unchanged over the one chunk list."""
         ctx = self.ctx
         d = ctx.stage(d)     # unchanged when it is aligned and has slack behind it; re-staged otherwise
-        cuts = ctx.chunk(d, self.cdc)
+        file_chunk = None
+        if files is None:
+            cuts = ctx.chunk(d, self.cdc)
+        else:
+            cuts, file_chunk = ctx.chunk_files(d, file_offsets(files, d.numel(), ctx), self.cdc)
         digests = ctx.digest(d, cuts)
         canon, first = ctx.dedup(digests)
         base = dblob = doffs = None
@@ -85,7 +95,8 @@ class Ingest:
             blob, offs = ctx.compress(d, cuts, sel, self.zdict, self.level)
         else:
             blob, offs = ctx.empty(0, torch.uint8), ctx.empty(1, torch.int64).zero_()
-        return IngestResult(cuts, digests, canon, first, sel, blob, offs, base=base, delta_blob=dblob, delta_offsets=doffs)
+        return IngestResult(cuts, digests, canon, first, sel, blob, offs, base=base, delta_blob=dblob, delta_offsets=doffs,
+                            file_chunk=file_chunk)
 
 
 @dataclass

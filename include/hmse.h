@@ -37,7 +37,7 @@ extern "C" {
 #define HMSE_E_NOMEM (-4)    /* scratch allocation failed                      */
 #define HMSE_E_NCCL (-5)     /* NCCL is missing or a collective failed (text in hmse_last_error) */
 
-#define HMSE_ABI_VERSION 2
+#define HMSE_ABI_VERSION 3
 
 typedef struct hmse_ctx hmse_ctx;
 
@@ -96,6 +96,17 @@ int hmse_compress_stats(hmse_ctx* ctx, uint64_t* out4, float* parse_ms_sum, uint
  * required capacity. */
 int hmse_chunk(hmse_ctx* ctx, const uint8_t* d_data, uint64_t n, const hmse_cdc_cfg* cfg,
                uint64_t* d_cuts, uint64_t cap, uint64_t* n_cuts, void* stream);
+
+/* Many independent streams in one call.  File f = d_data[d_file_off[f] : d_file_off[f+1]) is chunked on its own,
+ * exactly as hmse_chunk would chunk it in a buffer of its own (cuts at every file end; an empty file has no chunk).
+ * d_file_off[n_files+1] (device) starts at 0, never decreases and ends at n; d_data as for hmse_chunk (16-byte aligned).
+ * d_cuts receives one chunk list over the whole buffer (absolute offsets, start0 = 0); d_file_chunk[n_files+1] (device)
+ * = index of each file's first chunk, d_file_chunk[n_files] = *n_cuts.  n / min_size + n_files + 1 always suffices as
+ * cap; on HMSE_E_CAPACITY *n_cuts holds the capacity needed.  Bad offsets fail with HMSE_E_INVAL (checked on the
+ * device, nothing written outside the outputs).  Synchronises `stream`. */
+int hmse_chunk_files(hmse_ctx* ctx, const uint8_t* d_data, uint64_t n, const uint64_t* d_file_off, uint64_t n_files,
+                     const hmse_cdc_cfg* cfg, uint64_t* d_cuts, uint64_t cap, uint64_t* n_cuts,
+                     uint64_t* d_file_chunk, void* stream);
 
 /* Sharded stream, step 1: candidate scan of d_data[0:n_avail) into ctx scratch. */
 int hmse_chunk_scan(hmse_ctx* ctx, const uint8_t* d_data, uint64_t n_avail, const hmse_cdc_cfg* cfg,
