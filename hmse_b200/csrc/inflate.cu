@@ -85,10 +85,11 @@ struct BitReader {
 __device__ __forceinline__ uint32_t rev_bits(uint32_t code, uint32_t len) { return __brev(code) >> (32 - len); }
 
 // Builds the direct lookup + canonical arrays of one code from lens[0..n).  Collective over the warp.
-// Returns false if the lengths over-subscribe the code space (incomplete codes are accepted only in the forms
-// zlib accepts: a single code of length 1).
+// Accepts exactly the length sets zlib's inflate_table accepts: a complete code, a code with no symbols at all (a
+// symbol read from it is then an error), or - except for the code-length code (cl_code) - a single code of length 1.
+// Returns false on an over-subscribed or any other incomplete set.
 __device__ bool build_table(const uint8_t* lens, uint32_t n, uint16_t* tab, uint32_t tbits, uint16_t* sym, uint16_t* count,
-                            unsigned lane) {
+                            bool cl_code, unsigned lane) {
     for (uint32_t i = lane; i < (1u << tbits); i += 32) tab[i] = 0;
     if (lane < 16) count[lane] = 0;
     __syncwarp();
@@ -97,7 +98,7 @@ __device__ bool build_table(const uint8_t* lens, uint32_t n, uint16_t* tab, uint
     __syncwarp();
     // first code and first index of every length (every lane computes them: 15 steps)
     uint32_t first[16], offs[16];
-    uint32_t code = 0, idx = 0, used = 0;
+    uint32_t code = 0, idx = 0, max_len = 0;
     int left = 1;
     bool over = false;
     first[0] = offs[0] = 0;
@@ -110,10 +111,10 @@ __device__ bool build_table(const uint8_t* lens, uint32_t n, uint16_t* tab, uint
         offs[l] = idx;
         code = (code + c) << 1;
         idx += c;
-        used += c;
+        if (c) max_len = l;
     }
     if (over) return false;
-    if (left > 0 && !(used <= 1)) return false;   // incomplete set (zlib allows only the degenerate one-code case)
+    if (left > 0 && max_len != 0 && (cl_code || max_len != 1)) return false;   // incomplete
     // rank of a symbol inside its length class = symbols of the same length before it: chunks of 32 in order
     uint32_t seen[16];
 #pragma unroll
@@ -287,7 +288,7 @@ __global__ void __launch_bounds__(IW * 32) inflate_kernel(InfArgs a) {
                 if (lane < 19) T.lens[lane] = (uint8_t)my_cl;
                 __syncwarp();
                 uint16_t* clsym = T.lsym;   // scratch: rebuilt below
-                if (!build_table(T.lens, 19, T.cl_tab, 7, clsym, T.lcount, lane)) {
+                if (!build_table(T.lens, 19, T.cl_tab, 7, clsym, T.lcount, true, lane)) {
                     status = INF_BAD_BLOCK;
                     break;
                 }
@@ -349,8 +350,8 @@ __global__ void __launch_bounds__(IW * 32) inflate_kernel(InfArgs a) {
                     break;
                 }
             }
-            if (!build_table(T.lens, 288, T.lit, LBITS, T.lsym, T.lcount, lane) ||
-                !build_table(T.lens + 288, 32, T.dist, DBITS, T.dsym, T.dcount, lane)) {
+            if (!build_table(T.lens, 288, T.lit, LBITS, T.lsym, T.lcount, false, lane) ||
+                !build_table(T.lens + 288, 32, T.dist, DBITS, T.dsym, T.dcount, false, lane)) {
                 status = INF_BAD_BLOCK;
                 break;
             }
