@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libhmse_b200.so")
 
 HMSE_OK, HMSE_E_INVAL, HMSE_E_CAPACITY, HMSE_E_CUDA, HMSE_E_NOMEM, HMSE_E_NCCL = 0, -1, -2, -3, -4, -5
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 
 class HmseError(RuntimeError):
@@ -66,6 +66,9 @@ SIGNATURES = {
     "hmse_index_build_l4": (_I, [_P, _P, _P, _P, _U64, _U64, _P, _U64, _P, _P, _P, _P, _P, _P, _P, _U64, _PU64, _P]),
     "hmse_segment_copy": (_I, [_P, _P, _P, _P, _P, _U64, _P]),
     "hmse_inflate": (_I, [_P, _P, _P, _U64, _P, _U32, _P, _P, _P, _PU64, _P]),
+    "hmse_read_layout_bytes": (_U64, [_U64, _U64, _U64]),
+    "hmse_read_open": (_I, [_P, _P, _U64, _P, _U64, _U64, _P, _U64, _U64, _U64, _P, _U32, _P, _U64, _P]),
+    "hmse_read": (_I, [_P, _P, _U64, _U64, _U64, _P, _P, _P, _U32, _P, _U64, _P, _U64, _P, _PU64, _P, _PU64, _PU64, _P]),
     "hmse_minhash": (_I, [_P, _P, _U64, _P, _U64, _P, _U32, _P, _P]),
     "hmse_minhash_select": (_I, [_P, _P, _U64, _P, _P, _U64, _P, _U32, _P, _P]),
     "hmse_lsh_keys": (_I, [_P, _P, _U64, _U32, _U32, _P, _P]),

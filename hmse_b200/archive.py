@@ -1,7 +1,9 @@
 """The ingest result as a usable artefact: the spec's on-disk records (40-byte `ChunkIndex` entries,
 README.md:1264-1269; 8-byte pointer records, README.md:1312; the packed chunk store, README.md:1879-1887) in one
-container, written from the device results and restored through the device read path (hmse_inflate +
-hmse_segment_copy, README.md:1617-1675).
+container, written from the device results and read through the device read path (README.md:1617-1675): `Reader`
+opens an archive once (hmse_read_open checks the records and derives the layout on the device) and serves batches of
+byte ranges (hmse_read: every stored chunk and delta a batch needs is inflated / applied once, then the pieces are
+copied out); `restore` is one range per stream or per file.
 
 Container v1, little endian:
     0   magic b"HMSEARC1"
@@ -24,7 +26,8 @@ table after the chunk store and the delta store (which is empty, with n_delta ==
     ..  u64 n_files, u64 file_chunk[n_files + 1]     file f = chunks file_chunk[f] .. file_chunk[f+1]-1 (stream order)
 file_chunk starts at 0, never decreases and ends at n_chunks; an empty file has as many entries as any other.  The
 table holds indices only: file names, modes and times are not part of the container.  restore(files=[...]) rebuilds
-single files and inflates only the stored chunks (and delta bases) those files reference.
+single files and Reader.read(..., files=...) reads ranges inside them; both inflate only the stored chunks (and delta
+bases) the ranges reference.
 The v1 / v2 layout is restated for the tests in oracle/archive.py, v3 in tests/files_ref.py."""
 from __future__ import annotations
 
@@ -37,6 +40,7 @@ from typing import Optional
 import numpy as np
 import torch
 
+from . import _lib
 from .api import Context, default_context
 
 MAGIC = b"HMSEARC1"
@@ -177,150 +181,125 @@ def build(res, zdict: bytes, raw_bytes: Optional[int] = None, ctx: Optional[Cont
                    np.ascontiguousarray(store), int(raw_bytes), dstore, n_delta, fc)
 
 
+class Reader:
+    """An archive opened for random-access reads on the device (hmse_read_open / hmse_read).  The store, the delta
+    store, the dictionary, the index and the pointer records are copied to the device once, the records are checked
+    and the layout reads need is derived on the device; every `read` then serves a batch of byte ranges.  Raises
+    ValueError on a damaged archive (the failed check is named)."""
+
+    def __init__(self, ar: Archive, ctx: Optional[Context] = None):
+        ctx = ctx or default_context()
+        self.ctx, self.ar = ctx, ar
+        self.n, self.m, self.raw_bytes = ar.n_chunks, ar.n_unique, int(ar.raw_bytes)
+        self.n_delta = int(ar.n_delta) if ar.delta_store is not None else 0
+        self.zd = ctx.stage(ar.zdict)
+        self.store = ctx.stage(ar.store)
+        self.dstore = ctx.stage(ar.delta_store) if self.n_delta else None
+        index = ctx.stage(np.ascontiguousarray(ar.index).reshape(-1))
+        pointers = ctx.stage(np.ascontiguousarray(ar.pointers).reshape(-1))
+        lib = ctx.lib
+        nbytes = int(lib.hmse_read_layout_bytes(self.n, self.m, self.n_delta))
+        self.layout = ctx.empty(nbytes, torch.uint8)
+        rc = lib.hmse_read_open(ctx.h, index.data_ptr(), self.m, pointers.data_ptr(), self.n, int(ar.store.size),
+                                self.dstore.data_ptr() if self.n_delta else None, int(ar.delta_store.size) if self.n_delta else 0,
+                                self.n_delta, self.raw_bytes, self.zd.data_ptr() if len(ar.zdict) else None, len(ar.zdict),
+                                self.layout.data_ptr(), nbytes, ctx.stream)
+        if rc == _lib.HMSE_E_INVAL:
+            raise ValueError((lib.hmse_last_error(ctx.h) or b"").decode("utf-8", "replace"))
+        ctx.check(rc)
+        self.file_start = None    # raw offset of every file (v3), and the end of the stream
+        if ar.file_chunk is not None:
+            raw = ar.pointers[:, 6:8].copy().view("<u2").reshape(-1).astype(np.int64) + 1
+            start = np.concatenate([[0], np.cumsum(raw)])
+            self.file_start = start[ar.file_chunk.astype(np.int64)]
+
+    def file_size(self, f) -> np.ndarray:
+        return self.file_start[np.asarray(f) + 1] - self.file_start[np.asarray(f)]
+
+    def read(self, offsets, lengths, files=None, device_out: bool = False, stats: Optional[dict] = None):
+        """(data, off): the bytes of ranges [offsets[r], offsets[r] + lengths[r]) of the raw stream packed in request
+        order, data[off[r]:off[r+1]] for range r (numpy, or CUDA tensors with device_out).  files (v3): a file index per
+        range, offsets relative to the file, and every range must lie inside its file.  Raises IndexError for a bad
+        file index, ValueError for a range outside its file or the stream and for a range that needs a damaged chunk.
+        `stats` receives the streams inflated ("inflated"), the deltas applied ("deltas") and the raw bytes inflated
+        ("inflated_bytes") - every stored chunk and delta the batch needs counts once."""
+        ctx = self.ctx
+        to_np = lambda x: np.asarray(x.cpu().numpy() if isinstance(x, torch.Tensor) else x).reshape(-1)  # noqa: E731
+        off, ln = to_np(offsets), to_np(lengths)
+        if off.shape != ln.shape:
+            raise ValueError("offsets and lengths differ in size")
+        if (off.size and off.dtype.kind == "i" and (off < 0).any()) or (ln.size and ln.dtype.kind == "i" and (ln < 0).any()):
+            raise ValueError("negative offset or length")
+        off, ln = off.astype(np.uint64), ln.astype(np.uint64)
+        if files is not None:
+            if self.file_start is None:
+                raise ValueError("this archive has no file table (only v3 archives read by file)")
+            f = to_np(files).astype(np.int64)
+            if f.shape != off.shape:
+                raise ValueError("files and offsets differ in size")
+            nf = self.file_start.size - 1
+            if ((f < 0) | (f >= nf)).any():
+                raise IndexError("file index out of range (%d files)" % nf)
+            size = self.file_size(f).astype(np.uint64)
+            if ((ln > size) | (off > size - np.minimum(ln, size))).any():
+                raise ValueError("a range runs past the end of its file")
+            off = off + self.file_start[f].astype(np.uint64)
+        R = off.size
+        ends = np.concatenate([[np.uint64(0)], np.cumsum(ln, dtype=np.uint64)])
+        total = int(ends[-1]) if R else 0
+        if R and total < int(ln.max()):
+            raise ValueError("the ranges add up to more than 2^64 bytes")
+        ranges = ctx.stage_u64(np.stack([off, ln], axis=1).reshape(-1)) if R else ctx.empty(2, torch.int64)
+        out = ctx.empty(total + 64, torch.uint8)
+        out_off = ctx.empty(R + 1, torch.int64)
+        status = ctx.empty(max(R, 1), torch.int32)
+        got, bad, st4 = C.c_uint64(0), C.c_uint64(0), (C.c_uint64 * 4)()
+        rc = ctx.lib.hmse_read(ctx.h, self.layout.data_ptr(), self.n, self.m, self.n_delta, self.store.data_ptr(),
+                               self.dstore.data_ptr() if self.n_delta else None, self.zd.data_ptr() if self.zd.numel() else None,
+                               int(self.zd.numel()), ranges.data_ptr(), R, out.data_ptr(), total, out_off.data_ptr(),
+                               C.byref(got), status.data_ptr(), C.byref(bad), st4, ctx.stream)
+        if rc == _lib.HMSE_E_INVAL:
+            raise ValueError((ctx.lib.hmse_last_error(ctx.h) or b"").decode("utf-8", "replace"))
+        ctx.check(rc)
+        if bad.value:
+            first = int(torch.nonzero(status[:R])[0])
+            raise ValueError("%d ranges need a damaged chunk (first: range %d, status %d)" % (bad.value, first, int(status[first])))
+        if stats is not None:
+            stats.update(inflated=int(st4[0]), deltas=int(st4[1]), inflated_bytes=int(st4[2]))
+        data = out[:total]
+        if device_out:
+            return data, out_off
+        return data.cpu().numpy(), out_off.cpu().numpy().view(np.uint64)
+
+
 def restore(ar: Archive, ctx: Optional[Context] = None, device_out: bool = False, files=None, stats: Optional[dict] = None):
-    """The read path: the stored chunks needed are inflated once each on the device, and the output is rebuilt from the
-    pointer records.  files=None: returns the raw stream (numpy, or a CUDA tensor with device_out).  files = a sequence
-    of file indices (v3 archives): returns a list with the bytes of each requested file, in the order asked; only the
-    stored chunks those files reference, and the bases of their deltas, are gathered (hmse_segment_copy) and inflated.
-    `stats` (a dict) receives the number of zlib streams inflated ("inflated") and deltas applied ("deltas").  Raises
-    ValueError on a damaged archive."""
+    """The read path, through `Reader`: the stored chunks needed are inflated once each on the device, and the output is
+    rebuilt from the pointer records.  files=None: returns the raw stream (numpy, or a CUDA tensor with device_out) - one
+    range (0, raw_bytes).  files = a sequence of file indices (v3 archives): returns a list with the bytes of each
+    requested file, in the order asked - one range per file, so only the stored chunks those files reference, and the
+    bases of their deltas, are inflated.  `stats` (a dict) receives the number of zlib streams inflated ("inflated")
+    and deltas applied ("deltas").  Raises ValueError on a damaged archive."""
     ctx = ctx or default_context()
-    n, m = ar.n_chunks, ar.n_unique
     empty = lambda: ctx.empty(0, torch.uint8) if device_out else np.zeros(0, dtype=np.uint8)  # noqa: E731
-    if files is None:
-        rows = None
-    else:
+    if files is not None:
         if ar.file_chunk is None:
             raise ValueError("this archive has no file table (only v3 archives restore single files)")
         fsel = np.asarray(files, dtype=np.int64).reshape(-1)
         if ((fsel < 0) | (fsel >= ar.n_files)).any():
             raise IndexError("file index out of range (%d files)" % ar.n_files)
-        fc = ar.file_chunk.astype(np.int64)
-        lo, cnt = fc[fsel], fc[fsel + 1] - fc[fsel]
-        rows = np.repeat(lo - (np.cumsum(cnt) - cnt), cnt) + np.arange(int(cnt.sum()), dtype=np.int64)
     if stats is not None:
         stats.update(inflated=0, deltas=0)
-    if n == 0:
+    if ar.n_chunks == 0:
         return empty() if files is None else [empty() for _ in fsel]
-    idx = ar.index
-    lba_u = idx[:, 32:36].copy().view(np.uint32).reshape(-1).astype(np.int64)
-    clen = idx[:, 36:38].copy().view(np.uint16).reshape(-1).astype(np.int64)
-    p = ar.pointers
-    lba = p[:, 0:4].copy().view(np.uint32).reshape(-1).astype(np.int64)
-    off = p[:, 4:6].copy().view(np.uint16).reshape(-1).astype(np.int64)
-    raw = p[:, 6:8].copy().view(np.uint16).reshape(-1).astype(np.int64) + 1
-    pos = lba * 512 + off
-    is_delta = pos >= ar.store.size
-    if is_delta.any() and (ar.delta_store is None or not ar.n_delta):
-        raise ValueError("a pointer record addresses a delta store this archive does not have")
-    dpos_all = pos - ar.store.size      # DeltaChunk position of the chunks stored as deltas
-    pos = np.where(is_delta, 0, pos)    # (delta chunks are resolved below; slot 0 is a placeholder)
-    # store positions of the index entries: sector from the entry, exact byte from the running sum of lengths
-    upos = np.concatenate([[0], np.cumsum(clen)[:-1]])
-    if not np.array_equal(upos >> 9, lba_u) or int(upos[-1] + clen[-1]) != ar.store.size:
-        raise ValueError("index entries do not tile the chunk store")
-    slot = np.searchsorted(upos, pos)
-    if (slot >= m).any() or not np.array_equal(upos[slot], pos):
-        raise ValueError("a pointer record does not address a stored chunk")
-    # raw length of every unique chunk = raw length of any chunk pointing at it
-    ulen = np.zeros(m, dtype=np.int64)
-    ulen[slot[~is_delta]] = raw[~is_delta]
-    dinfo = None
-    rec = np.full(n, -1, dtype=np.int64)    # DeltaChunk record of every chunk stored as a delta
-    if is_delta.any():
-        # DeltaChunk headers: { u32 base slot, u16 base raw length - 1, u16 delta length }
-        ds = ar.delta_store
-        dpos, dinv = np.unique(dpos_all[is_delta], return_inverse=True)
-        if (dpos < 0).any() or (dpos + 8 > ds.size).any():
-            raise ValueError("a pointer record addresses outside the delta store")
-        hdr = ds[(dpos[:, None] + np.arange(8)[None, :])]
-        bslot = hdr[:, 0:4].copy().view("<u4").reshape(-1).astype(np.int64)
-        blen = hdr[:, 4:6].copy().view("<u2").reshape(-1).astype(np.int64) + 1
-        dlen = hdr[:, 6:8].copy().view("<u2").reshape(-1).astype(np.int64)
-        if (bslot >= m).any() or (dpos + 8 + dlen > ds.size).any():
-            raise ValueError("a DeltaChunk record is damaged")
-        traw = np.zeros(dpos.size, dtype=np.int64)
-        traw[dinv] = raw[is_delta]
-        if not np.array_equal(traw[dinv], raw[is_delta]):
-            raise ValueError("pointer records disagree about a delta chunk's length")
-        known = ulen[bslot] != 0
-        if not np.array_equal(ulen[bslot][known], blen[known]):
-            raise ValueError("a DeltaChunk record disagrees with the pointer records about its base's length")
-        ulen[bslot] = blen              # a base may be referenced by deltas only
-        dinfo = (dpos, bslot, blen, dlen, traw)
-        rec[is_delta] = dinv
-    if (ulen == 0).any() or not np.array_equal(ulen[slot[~is_delta]], raw[~is_delta]):
-        raise ValueError("pointer records disagree about a chunk's length")
-    if int(raw.sum()) != ar.raw_bytes:
-        raise ValueError("pointer records do not add up to the stream length")
-    if rows is not None and rows.size == 0:
-        return [empty() for _ in fsel]
-    # what the requested chunks need: their stored chunks, their DeltaChunk records and those records' bases
-    if rows is None:
-        rows = np.arange(n, dtype=np.int64)
-        need_r = np.arange(dinfo[0].size, dtype=np.int64) if dinfo is not None else np.zeros(0, dtype=np.int64)
-        need_u = np.arange(m, dtype=np.int64)
-    else:
-        rd = is_delta[rows]
-        need_r = np.unique(rec[rows[rd]])
-        need_u = np.unique(np.concatenate([slot[rows[~rd]], dinfo[1][need_r] if dinfo is not None else []]).astype(np.int64))
-    u_at = np.full(m, -1, dtype=np.int64)
-    u_at[need_u] = np.arange(need_u.size)
-    zd = ctx.stage(ar.zdict)
-    store = ctx.stage(ar.store)
-    if need_u.size == m:
-        blob, offs = store, ctx.stage_u64(np.concatenate([upos, [ar.store.size]]).astype(np.uint64))
-    else:
-        # gather the streams of the needed chunks into one packed blob
-        goff = np.concatenate([[0], np.cumsum(clen[need_u])]).astype(np.uint64)
-        blob = ctx.empty(int(goff[-1]) + 64, torch.uint8)
-        g_src, offs = ctx.stage_u64(upos[need_u].astype(np.uint64)), ctx.stage_u64(goff)   # named: they must outlive the call
-        if need_u.size:
-            ctx.check(ctx.lib.hmse_segment_copy(ctx.h, store.data_ptr(), g_src.data_ptr(), blob.data_ptr(), offs.data_ptr(),
-                                                need_u.size, ctx.stream))
-    uo = np.concatenate([[0], np.cumsum(ulen[need_u])]).astype(np.uint64)
-    uniq, status, bad = ctx.inflate(blob, offs, ctx.stage_u64(uo), zd)
-    if bad:
-        raise ValueError("%d stored chunks failed to inflate (first: %d)" % (bad, int(need_u[int(torch.nonzero(status)[0])])))
-    if stats is not None:
-        stats.update(inflated=int(need_u.size), deltas=int(need_r.size))
-    rows_d = is_delta[rows]
-    src = np.zeros(rows.size, dtype=np.uint64)
-    src[~rows_d] = uo[:-1][u_at[slot[rows[~rows_d]]]]
-    if need_r.size:
-        dpos, bslot, blen, dlen, traw = (x[need_r] for x in dinfo)
-        r_at = np.full(dinfo[0].size, -1, dtype=np.int64)
-        r_at[need_r] = np.arange(need_r.size)
-        doff = np.concatenate([[0], np.cumsum(dlen)]).astype(np.uint64)
-        dsd = ctx.stage(ar.delta_store)
-        # gather the delta bytes of the records (they sit behind their 8-byte headers) into one packed blob
-        dblob = ctx.empty(int(doff[-1]) + 64, torch.uint8)[:int(doff[-1])]
-        t_src, t_dst = ctx.stage_u64((dpos + 8).astype(np.uint64)), ctx.stage_u64(doff)   # named: they must outlive the call
-        ctx.check(ctx.lib.hmse_segment_copy(ctx.h, dsd.data_ptr(), t_src.data_ptr(), dblob.data_ptr(), t_dst.data_ptr(),
-                                            dpos.size, ctx.stream))
-        to = np.concatenate([[0], np.cumsum(traw)]).astype(np.uint64)
-        bl = torch.from_numpy(blen.astype(np.uint32).view(np.int32).copy()).to(ctx.tdev)
-        tout, dstatus, dbad = ctx.delta_apply(dblob, t_dst, uniq, ctx.stage_u64(uo[:-1][u_at[bslot]].astype(np.uint64)), bl,
-                                              ctx.stage_u64(to))
-        if dbad:
-            raise ValueError("%d deltas failed to apply (first: %d)" % (dbad, int(torch.nonzero(dstatus)[0])))
-        total_u = int(uo[-1])
-        both = ctx.empty(total_u + int(to[-1]) + 64, torch.uint8)
-        both[:total_u].copy_(uniq)
-        both[total_u:total_u + int(to[-1])].copy_(tout)
-        uniq = both
-        src[rows_d] = np.uint64(total_u) + to[:-1][r_at[rec[rows[rows_d]]]]
-    out_len = raw[rows]
-    total = int(out_len.sum())
-    out = ctx.empty(total + 64, torch.uint8)[:total]
-    src_off = ctx.stage_u64(src)
-    dst = np.concatenate([[0], np.cumsum(out_len)]).astype(np.uint64)
-    dst_off = ctx.stage_u64(dst)
-    if rows.size:
-        ctx.check(ctx.lib.hmse_segment_copy(ctx.h, uniq.data_ptr(), src_off.data_ptr(), out.data_ptr(), dst_off.data_ptr(),
-                                            rows.size, ctx.stream))
+    rd = Reader(ar, ctx)
+    st = {}
     if files is None:
-        return out if device_out else out.cpu().numpy()
-    res = out if device_out else out.cpu().numpy()
-    ends = dst[np.cumsum(cnt)].astype(np.int64)
-    return [res[int(a):int(b)] for a, b in zip(np.concatenate([[0], ends[:-1]]), ends)]
+        data, _ = rd.read([0], [rd.raw_bytes], device_out=device_out, stats=st)
+    else:
+        data, off = rd.read(np.zeros(fsel.size, dtype=np.uint64), rd.file_size(fsel), files=fsel, device_out=device_out, stats=st)
+        off = off.cpu().numpy().view(np.uint64) if isinstance(off, torch.Tensor) else off
+    if stats is not None:
+        stats.update(inflated=st["inflated"], deltas=st["deltas"])
+    if files is None:
+        return data
+    return [data[int(a):int(b)] for a, b in zip(off[:-1], off[1:])]

@@ -39,6 +39,10 @@ enum HmseSlot {
     SLOT_COMM_SMALL,    // counts / exits travelling through the all-gathers
     SLOT_COMM_SEND,     // records (dedup) or key columns (LSH) grouped by destination rank
     SLOT_COMM_RECV,     // what arrives, the owner's answers, the replies
+    SLOT_READ_OPEN,     // record-number flags over delta-store positions, error word (hmse_read_open)
+    SLOT_READ_PLAN,     // per-range lengths / first chunks / piece counts, need marks and their scans (hmse_read)
+    SLOT_READ_WORK,     // need lists, per-stream statuses, piece offsets, gathered delta bytes
+    SLOT_READ_DATA,     // the inflated stored chunks and applied deltas of one hmse_read batch
     SLOT_COUNT
 };
 
@@ -47,7 +51,8 @@ constexpr int HMSE_PARSE_EVENTS = 128;
 constexpr int HMSE_MAX_WORLD = 32;          // ranks per communicator (the counts matrix must fit the mailbox)
 constexpr size_t HMSE_MAILBOX_BYTES = 16384;
 enum HmseTimer {
-    HT_SCAN = 0, HT_RESOLVE, HT_SHA, HT_DEDUP, HT_DEFLATE, HT_PACK, HT_MINHASH, HT_LSH, HT_INFLATE, HT_DELTA, HT_EXCHANGE, HT_COUNT
+    HT_SCAN = 0, HT_RESOLVE, HT_SHA, HT_DEDUP, HT_DEFLATE, HT_PACK, HT_MINHASH, HT_LSH, HT_INFLATE, HT_DELTA, HT_EXCHANGE,
+    HT_READ_PLAN, HT_READ_COPY, HT_COUNT
 };
 
 struct hmse_ctx {
@@ -133,6 +138,13 @@ int hmse_exclusive_scan_u64(hmse_ctx* ctx, const uint64_t* d_in, uint64_t* d_out
 // (the compressed blobs of the previous piece, when the caller streams), a store from an SM does not.
 // Copies n32 32-bit words from d_src to mailbox word `word32` (4-byte units).  Asynchronous on `stream`.
 int hmse_mail(hmse_ctx* ctx, uint32_t word32, const void* d_src, uint32_t n32, cudaStream_t stream);
+
+// hmse_inflate without the host round trips: streams j = d_blob[d_begin[j] : d_end[j]) (d_end null: d_begin[j+1]),
+// the dictionary's Adler-32 given by the caller.  Asynchronous on `stream`.
+int hmse_inflate_ranges(hmse_ctx* ctx, const uint8_t* d_blob, const uint64_t* d_begin, const uint64_t* d_end, uint64_t m,
+                        const uint8_t* d_zdict, uint32_t dict_len, uint32_t dict_adler, uint8_t* d_out,
+                        const uint64_t* d_out_offsets, uint32_t* d_status, cudaStream_t stream);
+uint32_t hmse_adler32_host(const uint8_t* d, size_t n);
 
 // hmse_dedup_partition without the host round trip: d_counts[world] (device) receives the records per owner.
 int hmse_dedup_partition_dev(hmse_ctx* ctx, const uint8_t* d_digests, uint64_t n, uint64_t id_base, uint32_t world,

@@ -186,7 +186,8 @@ __constant__ uint8_t c_clorder[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4, 1
 
 struct InfArgs {
     const uint8_t* blob;
-    const uint64_t* offs;       // [m+1]
+    const uint64_t* offs;       // [m+1]; with offs_end: [m], stream j = blob[offs[j] : offs_end[j])
+    const uint64_t* offs_end;   // null: stream j = blob[offs[j] : offs[j+1])
     uint64_t m;
     const uint8_t* dict;
     uint32_t dict_len, dict_adler;
@@ -207,7 +208,7 @@ __global__ void __launch_bounds__(IW * 32) inflate_kernel(InfArgs a) {
         if (j >= a.m) break;
         // the offsets come from the caller (an archive that may be damaged): a stream or an output range that runs
         // backwards, or an output range beyond 32 bits, is reported and nothing is read or written for it
-        const uint64_t o0 = a.offs[j], o1 = a.offs[j + 1], q0 = a.out_offs[j], q1 = a.out_offs[j + 1];
+        const uint64_t o0 = a.offs[j], o1 = a.offs_end ? a.offs_end[j] : a.offs[j + 1], q0 = a.out_offs[j], q1 = a.out_offs[j + 1];
         if (o1 < o0 || q1 < q0 || q1 - q0 > 0xFFFFFFFFull) {
             if (lane == 0) a.status[j] = o1 < o0 ? INF_BAD_HEADER : INF_OVERRUN;
             continue;
@@ -456,6 +457,38 @@ __global__ void count_bad_kernel(const uint32_t* __restrict__ status, uint64_t m
 
 }  // namespace
 
+// Streams j = d_blob[d_begin[j] : d_end[j]) (d_end null: d_begin[j+1]), the DICTID given by the caller; no host round
+// trip.  hmse_read inflates the stored chunks it needs in place in the chunk store through this form.
+int hmse_inflate_ranges(hmse_ctx* ctx, const uint8_t* d_blob, const uint64_t* d_begin, const uint64_t* d_end, uint64_t m,
+                        const uint8_t* d_zdict, uint32_t dict_len, uint32_t dict_adler, uint8_t* d_out,
+                        const uint64_t* d_out_offsets, uint32_t* d_status, cudaStream_t st) {
+    if (m == 0) return HMSE_OK;
+    HMSE_SCRATCH(ctx, misc, unsigned long long*, SLOT_INFLATE_MISC, 64);
+    HMSE_CUDA(ctx, cudaMemsetAsync(misc, 0, 64, st));
+    InfArgs a;
+    a.blob = d_blob;
+    a.offs = d_begin;
+    a.offs_end = d_end;
+    a.m = m;
+    a.dict = d_zdict;
+    a.dict_len = dict_len;
+    a.dict_adler = dict_adler;
+    a.out = d_out;
+    a.out_offs = d_out_offsets;
+    a.status = d_status;
+    a.counter = (unsigned int*)(misc + 1);
+    const uint64_t want = div_up64(m, IW);
+    const uint64_t cap = (uint64_t)ctx->sm_count * 8;
+    HT_BEGIN(ctx, HT_INFLATE, st);
+    KL(ctx);
+    inflate_kernel<<<(unsigned)(want < cap ? want : cap), IW * 32, 0, st>>>(a);
+    HMSE_LAUNCH_CHECK(ctx);
+    HT_END(ctx, HT_INFLATE, st);
+    return HMSE_OK;
+}
+
+uint32_t hmse_adler32_host(const uint8_t* d, size_t n) { return host_adler32(d, n); }
+
 HMSE_API int hmse_inflate(hmse_ctx* ctx, const uint8_t* d_blob, const uint64_t* d_offsets, uint64_t m, const uint8_t* d_zdict,
                           uint32_t dict_len, uint8_t* d_out, const uint64_t* d_out_offsets, uint32_t* d_status,
                           uint64_t* n_bad, void* stream) {
@@ -474,27 +507,11 @@ HMSE_API int hmse_inflate(hmse_ctx* ctx, const uint8_t* d_blob, const uint64_t* 
         HMSE_CUDA(ctx, cudaStreamSynchronize(st));
         dict_adler = host_adler32(tmp, dict_len);
     }
-    HMSE_SCRATCH(ctx, misc, unsigned long long*, SLOT_INFLATE_MISC, 64);
-    HMSE_CUDA(ctx, cudaMemsetAsync(misc, 0, 64, st));
-    InfArgs a;
-    a.blob = d_blob;
-    a.offs = d_offsets;
-    a.m = m;
-    a.dict = d_zdict;
-    a.dict_len = dict_len;
-    a.dict_adler = dict_adler;
-    a.out = d_out;
-    a.out_offs = d_out_offsets;
-    a.status = d_status;
-    a.counter = (unsigned int*)(misc + 1);
-    const uint64_t want = div_up64(m, IW);
-    const uint64_t cap = (uint64_t)ctx->sm_count * 8;
-    HT_BEGIN(ctx, HT_INFLATE, st);
-    KL(ctx);
-    inflate_kernel<<<(unsigned)(want < cap ? want : cap), IW * 32, 0, st>>>(a);
-    HMSE_LAUNCH_CHECK(ctx);
-    HT_END(ctx, HT_INFLATE, st);
+    if (int rc = hmse_inflate_ranges(ctx, d_blob, d_offsets, nullptr, m, d_zdict, dict_len, dict_adler, d_out, d_out_offsets,
+                                     d_status, st))
+        return rc;
     if (n_bad) {
+        HMSE_SCRATCH(ctx, misc, unsigned long long*, SLOT_INFLATE_MISC, 64);
         KL(ctx);
         count_bad_kernel<<<(unsigned)div_up64(m, 256), 256, 0, st>>>(d_status, m, misc);
         HMSE_LAUNCH_CHECK(ctx);

@@ -37,7 +37,7 @@ extern "C" {
 #define HMSE_E_NOMEM (-4)    /* scratch allocation failed                      */
 #define HMSE_E_NCCL (-5)     /* NCCL is missing or a collective failed (text in hmse_last_error) */
 
-#define HMSE_ABI_VERSION 3
+#define HMSE_ABI_VERSION 4
 
 typedef struct hmse_ctx hmse_ctx;
 
@@ -78,6 +78,8 @@ int hmse_guard_check(hmse_ctx* ctx);
 #define HMSE_T_INFLATE 8
 #define HMSE_T_DELTA 9
 #define HMSE_T_EXCHANGE 10 /* the NCCL part of the last hmse_chunk_sharded / hmse_dedup_global / hmse_lsh_exchange */
+#define HMSE_T_READ_PLAN 11 /* hmse_read steps 1-4: range checks, locate, pieces, need lists and their scans */
+#define HMSE_T_READ_COPY 12 /* hmse_read: the pieces copied into the output, statuses folded per range */
 int hmse_timing(hmse_ctx* ctx, int enable);
 int hmse_timing_ms(hmse_ctx* ctx, int id, float* ms);
 /* Kernels launched through this ctx since hmse_create. */
@@ -283,6 +285,47 @@ int hmse_index_build_l4(hmse_ctx* ctx, const uint8_t* d_digests, const int64_t* 
  * entries, d_src_off n; d_src needs 4 readable bytes after its last segment). */
 int hmse_segment_copy(hmse_ctx* ctx, const uint8_t* d_src, const uint64_t* d_src_off, uint8_t* d_dst,
                       const uint64_t* d_dst_off, uint64_t n, void* stream);
+
+/* ---- Random-access reads: byte ranges of an archive's raw stream, many per call, planned on the device
+ *      (the spec's read path, README.md:1617-1675, from pointer records to chunks, for ranges instead of whole
+ *      streams).  An archive is opened once (hmse_read_open derives a device layout the caller owns) and read many
+ *      times; the library keeps no per-archive state, so one ctx serves any number of open archives. ---------------- */
+
+/* Bytes of the device layout buffer for an archive of n chunks, m stored chunks and n_delta DeltaChunk records. */
+uint64_t hmse_read_layout_bytes(uint64_t n, uint64_t m, uint64_t n_delta);
+
+/* Checks the records of an archive on the device and derives what reads need into d_layout (8-byte aligned,
+ * layout_bytes >= hmse_read_layout_bytes(n, m, n_delta)): the raw offset of every chunk, the stored slot or DeltaChunk
+ * record of every chunk, the store position and raw length of every stored chunk, the base, lengths and position of
+ * every record, and the Adler-32 of the dictionary.  d_index = m 40-byte ChunkIndex entries (4-byte aligned),
+ * d_pointers = n 8-byte pointer records (8-byte aligned), n_delta == 0: no delta store.  Fails with HMSE_E_INVAL, the
+ * failed check named, when (1) the index entries do not tile the store, (2) a pointer below store_bytes does not
+ * address the start of a stored chunk, (3) a pointer at or above store_bytes has no delta store, or its record header
+ * or delta bytes lie outside it, or its base slot is >= m, (4) two references to one stored chunk or one record
+ * disagree on its raw length (a record's base length counts as a reference to its base), (5) a stored chunk has no
+ * known raw length, (6) the raw lengths do not add up to raw_bytes.  Synchronises `stream`. */
+int hmse_read_open(hmse_ctx* ctx, const uint8_t* d_index, uint64_t m, const uint8_t* d_pointers, uint64_t n,
+                   uint64_t store_bytes, const uint8_t* d_delta_store, uint64_t delta_store_bytes, uint64_t n_delta,
+                   uint64_t raw_bytes, const uint8_t* d_zdict, uint32_t dict_len,
+                   void* d_layout, uint64_t layout_bytes, void* stream);
+
+/* R ranges d_ranges[r] = {offset, length} of the raw stream -> d_out[d_out_off[r] : d_out_off[r+1]) (d_out_off written,
+ * packed in request order).  n, m, n_delta: those given to hmse_read_open for d_layout (a mismatch is HMSE_E_INVAL).
+ * d_store / d_delta_store / d_zdict: the buffers the layout was opened on; the stores need 16 readable bytes after
+ * their end.  Ranges may be empty, overlap, repeat and come in any order.  A range past raw_bytes (or one whose
+ * offset + length overflows) fails the call with HMSE_E_INVAL before anything is written.  *total (host) = bytes of
+ * all ranges; on HMSE_E_CAPACITY it holds the out_cap needed and nothing is written.  Every stored chunk and
+ * DeltaChunk record the batch needs is inflated / applied exactly once, whatever the number of ranges that touch it.
+ * d_status[r] = 0, else the hmse_inflate code (1-6) of a stored chunk the range needs, or 16 + the hmse_delta_apply
+ * code (1-5) of a delta it needs (the largest code when several fail); a failed range never causes writes outside its
+ * own output range, and ranges that need no damaged chunk are correct.  *n_bad (host) = ranges with a non-zero
+ * status.  stats4 (host, may be null) = {streams inflated, deltas applied, raw bytes inflated, pieces}.  Two host
+ * round trips (the sizes, then n_bad); the number of kernels does not depend on R, n or the ranges.  Synchronises
+ * `stream`. */
+int hmse_read(hmse_ctx* ctx, const void* d_layout, uint64_t n, uint64_t m, uint64_t n_delta, const uint8_t* d_store,
+              const uint8_t* d_delta_store, const uint8_t* d_zdict, uint32_t dict_len, const uint64_t* d_ranges,
+              uint64_t R, uint8_t* d_out, uint64_t out_cap, uint64_t* d_out_off, uint64_t* total, uint32_t* d_status,
+              uint64_t* n_bad, uint64_t* stats4, void* stream);
 
 /* ---- L4 similarity: replaces minhash_compute (README.md:2578-2597) and LSH banding
  *      (README.md:2231-2235). -------------------------------------------------------------- */
