@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libhmse_b200.so")
 
 HMSE_OK, HMSE_E_INVAL, HMSE_E_CAPACITY, HMSE_E_CUDA, HMSE_E_NOMEM, HMSE_E_NCCL = 0, -1, -2, -3, -4, -5
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 
 class HmseError(RuntimeError):
@@ -22,6 +22,11 @@ class CdcCfg(C.Structure):
     _fields_ = [("min_size", C.c_uint32), ("avg_size", C.c_uint32), ("max_size", C.c_uint32),
                 ("reserved", C.c_uint32), ("mask_s", C.c_uint64), ("mask_l", C.c_uint64),
                 ("gear", C.c_uint64 * 256)]
+
+
+class ComposeSrc(C.Structure):
+    _fields_ = [("d_layout", C.c_void_p), ("d_index", C.c_void_p), ("d_pointers", C.c_void_p), ("d_store", C.c_void_p),
+                ("d_delta_store", C.c_void_p), ("n", C.c_uint64), ("m", C.c_uint64), ("n_delta", C.c_uint64)]
 
 
 class CorpusCfg(C.Structure):
@@ -69,6 +74,7 @@ SIGNATURES = {
     "hmse_read_layout_bytes": (_U64, [_U64, _U64, _U64]),
     "hmse_read_open": (_I, [_P, _P, _U64, _P, _U64, _U64, _P, _U64, _U64, _U64, _P, _U32, _P, _U64, _P]),
     "hmse_read": (_I, [_P, _P, _U64, _U64, _U64, _P, _P, _P, _U32, _P, _U64, _P, _U64, _P, _PU64, _P, _PU64, _PU64, _P]),
+    "hmse_compose": (_I, [_P, C.POINTER(ComposeSrc), _U32, _P, _U64, _U64, _P, _P, _U64, _P, _U64, _P, _U64, _PU64, _P]),
     "hmse_minhash": (_I, [_P, _P, _U64, _P, _U64, _P, _U32, _P, _P]),
     "hmse_minhash_select": (_I, [_P, _P, _U64, _P, _P, _U64, _P, _U32, _P, _P]),
     "hmse_lsh_keys": (_I, [_P, _P, _U64, _U32, _U32, _P, _P]),

@@ -3,7 +3,9 @@ README.md:1264-1269; 8-byte pointer records, README.md:1312; the packed chunk st
 container, written from the device results and read through the device read path (README.md:1617-1675): `Reader`
 opens an archive once (hmse_read_open checks the records and derives the layout on the device) and serves batches of
 byte ranges (hmse_read: every stored chunk and delta a batch needs is inflated / applied once, then the pieces are
-copied out); `restore` is one range per stream or per file.
+copied out); `restore` is one range per stream or per file; `compose` turns files of several archives into one archive
+on the device (hmse_compose: stored chunks deduplicated across sources by digest, streams and records copied, nothing
+inflated).
 
 Container v1, little endian:
     0   magic b"HMSEARC1"
@@ -183,8 +185,9 @@ def build(res, zdict: bytes, raw_bytes: Optional[int] = None, ctx: Optional[Cont
 
 class Reader:
     """An archive opened for random-access reads on the device (hmse_read_open / hmse_read).  The store, the delta
-    store, the dictionary, the index and the pointer records are copied to the device once, the records are checked
-    and the layout reads need is derived on the device; every `read` then serves a batch of byte ranges.  Raises
+    store, the dictionary, the index and the pointer records are copied to the device once (and kept: `compose` reads
+    them), the records are checked and the layout reads need is derived on the device; every `read` then serves a batch
+    of byte ranges.  Raises
     ValueError on a damaged archive (the failed check is named)."""
 
     def __init__(self, ar: Archive, ctx: Optional[Context] = None):
@@ -195,12 +198,12 @@ class Reader:
         self.zd = ctx.stage(ar.zdict)
         self.store = ctx.stage(ar.store)
         self.dstore = ctx.stage(ar.delta_store) if self.n_delta else None
-        index = ctx.stage(np.ascontiguousarray(ar.index).reshape(-1))
-        pointers = ctx.stage(np.ascontiguousarray(ar.pointers).reshape(-1))
+        self.index = ctx.stage(np.ascontiguousarray(ar.index).reshape(-1))
+        self.pointers = ctx.stage(np.ascontiguousarray(ar.pointers).reshape(-1))
         lib = ctx.lib
         nbytes = int(lib.hmse_read_layout_bytes(self.n, self.m, self.n_delta))
         self.layout = ctx.empty(nbytes, torch.uint8)
-        rc = lib.hmse_read_open(ctx.h, index.data_ptr(), self.m, pointers.data_ptr(), self.n, int(ar.store.size),
+        rc = lib.hmse_read_open(ctx.h, self.index.data_ptr(), self.m, self.pointers.data_ptr(), self.n, int(ar.store.size),
                                 self.dstore.data_ptr() if self.n_delta else None, int(ar.delta_store.size) if self.n_delta else 0,
                                 self.n_delta, self.raw_bytes, self.zd.data_ptr() if len(ar.zdict) else None, len(ar.zdict),
                                 self.layout.data_ptr(), nbytes, ctx.stream)
@@ -303,3 +306,90 @@ def restore(ar: Archive, ctx: Optional[Context] = None, device_out: bool = False
     if files is None:
         return data
     return [data[int(a):int(b)] for a, b in zip(off[:-1], off[1:])]
+
+
+def compose(parts, ctx: Optional[Context] = None, stats: Optional[dict] = None) -> Archive:
+    """One v3 archive from files of several archives (hmse_compose): `parts` is a list of (source, files), a source an
+    `Archive` (opened for this call) or a `Reader` (opened once, for many calls), files None for every file of the source
+    (a v1 / v2 source is one file: its whole stream) or a list of file indices of a v3 source, in any order, repeats
+    allowed.  File j of the result is the j-th file selected.  Stored chunks are numbered by first reference in the
+    output stream and stored once per SHA-256 digest across sources, and their zlib streams and DeltaChunk records are
+    copied without inflating anything: for sources without deltas the result is byte for byte the archive one
+    `Ingest.run(files=...)` + `build` of the selected files, in that order, would write.  DeltaChunk records are not
+    deduplicated across sources (the container stores no digest for them).  Every part is a source of its own, even
+    when one archive appears in several parts.  `stats` receives "stored_referenced" (stored chunks referenced, before
+    the digest dedup), "stored", "deduplicated", "records", "store_bytes" and "delta_store_bytes".  Raises ValueError
+    for sources whose dictionaries differ, `files` on a source without a file table, an output of more than 2^32 - 2
+    chunks (before any device work) or a store of 2 TiB or more, and IndexError for a file index out of range."""
+    ctx = ctx or default_context()
+    parts = list(parts)
+    ars = [src.ar if isinstance(src, Reader) else src for src, _ in parts]
+    zd = bytes(ars[0].zdict) if ars else b""
+    if any(bytes(a.zdict) != zd for a in ars):
+        raise ValueError("the sources' dictionaries differ")
+    runs, sizes = [], []
+    for p, (a, (_, files)) in enumerate(zip(ars, parts)):
+        raw = a.pointers[:, 6:8].copy().view("<u2").reshape(-1).astype(np.int64) + 1
+        cstart = np.concatenate([[0], np.cumsum(raw)])
+        if files is None:
+            fc = a.file_chunk.astype(np.int64) if a.file_chunk is not None else np.array([0, a.n_chunks], dtype=np.int64)
+            f = np.arange(fc.size - 1)
+        else:
+            if a.file_chunk is None:
+                raise ValueError("part %d: the source has no file table (only v3 sources select files)" % p)
+            fc = a.file_chunk.astype(np.int64)
+            f = np.asarray(files, dtype=np.int64).reshape(-1)
+            if ((f < 0) | (f >= fc.size - 1)).any():
+                raise IndexError("part %d: file index out of range (%d files)" % (p, fc.size - 1))
+        first, cnt = fc[f], fc[f + 1] - fc[f]
+        runs.append(np.stack([np.full(f.size, p), first, cnt], axis=1))
+        sizes.append(cstart[fc[f + 1]] - cstart[first])
+    runs = np.concatenate(runs) if runs else np.zeros((0, 3), dtype=np.int64)
+    sizes = np.concatenate(sizes) if sizes else np.zeros(0, dtype=np.int64)
+    file_chunk = np.concatenate([[0], np.cumsum(runs[:, 2])]).astype(np.uint64)
+    n_out = int(file_chunk[-1])
+    if n_out > 0xFFFFFFFE:
+        raise ValueError("the output would hold %d chunks (at most 2^32 - 2)" % n_out)
+    runs = runs[runs[:, 2] > 0]
+    used = sorted(set(int(p) for p in runs[:, 0]))   # parts with chunks in the output: only these are opened
+    empty = np.zeros((0, 40), dtype=np.uint8)
+    if stats is not None:
+        stats.update(stored_referenced=0, stored=0, deduplicated=0, records=0, store_bytes=0, delta_store_bytes=0)
+    if n_out == 0:
+        return Archive(zd, empty, np.zeros((0, 8), dtype=np.uint8), np.zeros(0, dtype=np.uint8), 0, None, 0, file_chunk)
+    opened = {}
+    for p in used:
+        src = parts[p][0]
+        if isinstance(src, Reader):
+            opened.setdefault(id(src), src)
+        elif id(src) not in opened:
+            opened[id(src)] = Reader(src, ctx)
+    readers = [opened[id(parts[p][0])] for p in used]
+    slot = {p: k for k, p in enumerate(used)}
+    runs[:, 0] = [slot[int(p)] for p in runs[:, 0]]
+    descs = (_lib.ComposeSrc * len(readers))()
+    for d, rd in zip(descs, readers):
+        d.d_layout, d.d_index, d.d_pointers = rd.layout.data_ptr(), rd.index.data_ptr(), rd.pointers.data_ptr()
+        d.d_store, d.d_delta_store = rd.store.data_ptr(), rd.dstore.data_ptr() if rd.n_delta else None
+        d.n, d.m, d.n_delta = rd.n, rd.m, rd.n_delta
+    sb = sum(int(rd.ar.store.size) for rd in readers)
+    dsb = sum(int(rd.ar.delta_store.size) for rd in readers if rd.n_delta)
+    icap = min(n_out, sum(rd.m for rd in readers))
+    d_runs = ctx.stage_u64(runs.reshape(-1))
+    ptrs = ctx.empty(8 * n_out, torch.uint8)
+    index = ctx.empty(max(icap, 1) * 40, torch.uint8)
+    store = ctx.empty(max(sb, 1), torch.uint8)
+    dstore = ctx.empty(max(dsb, 1), torch.uint8)
+    out6 = (C.c_uint64 * 6)()
+    rc = ctx.lib.hmse_compose(ctx.h, descs, len(readers), d_runs.data_ptr(), runs.shape[0], n_out, ptrs.data_ptr(),
+                              index.data_ptr(), icap, store.data_ptr(), sb, dstore.data_ptr(), dsb, out6, ctx.stream)
+    if rc == _lib.HMSE_E_INVAL:
+        raise ValueError((ctx.lib.hmse_last_error(ctx.h) or b"").decode("utf-8", "replace"))
+    ctx.check(rc)
+    _, cand, kept, sbytes, recs, dbytes = (int(x) for x in out6)
+    if stats is not None:
+        stats.update(stored_referenced=cand, stored=kept, deduplicated=cand - kept, records=recs, store_bytes=sbytes,
+                     delta_store_bytes=dbytes)
+    return Archive(zd, index[:kept * 40].cpu().numpy().reshape(kept, 40), ptrs.cpu().numpy().reshape(n_out, 8),
+                   store[:sbytes].cpu().numpy(), int(sizes.sum()), dstore[:dbytes].cpu().numpy() if recs else None, recs,
+                   file_chunk)

@@ -57,12 +57,14 @@ __global__ void index_kernel(const uint8_t* __restrict__ digests, const uint64_t
     e[9] = (uint32_t)(len & 0xFFFF) | (rc << 16);
 }
 
-// dst[dst_off[i] .. dst_off[i+1]) = src[src_off[i] .. + the same length): one CTA per segment at a time.
+// dst[dst_off[i] .. dst_off[i+1]) = src[src_off[i] .. + the same length): one CTA per segment at a time.  GATHER: src_off[i]
+// is the segment's own source address (segments from several buffers), src is unused.
+template <bool GATHER>
 __global__ void __launch_bounds__(256) segment_copy_kernel(const uint8_t* __restrict__ src, const uint64_t* __restrict__ src_off,
                                                            uint8_t* __restrict__ dst, const uint64_t* __restrict__ dst_off,
                                                            uint64_t n) {
     for (uint64_t i = blockIdx.x; i < n; i += gridDim.x) {
-        const uint8_t* s = src + src_off[i];
+        const uint8_t* s = GATHER ? reinterpret_cast<const uint8_t*>(src_off[i]) : src + src_off[i];
         uint8_t* d = dst + dst_off[i];
         const uint64_t len = dst_off[i + 1] - dst_off[i];
         // head bytes until d is 4-aligned, then words assembled from the (arbitrarily aligned) source
@@ -257,7 +259,16 @@ HMSE_API int hmse_segment_copy(hmse_ctx* ctx, const uint8_t* d_src, const uint64
     if (!d_src || !d_src_off || !d_dst || !d_dst_off) HMSE_FAIL(ctx, HMSE_E_INVAL, "hmse_segment_copy: null pointer");
     const uint64_t cap = (uint64_t)ctx->sm_count * 16;
     KL(ctx);
-    segment_copy_kernel<<<(unsigned)(n < cap ? n : cap), 256, 0, (cudaStream_t)stream>>>(d_src, d_src_off, d_dst, d_dst_off, n);
+    segment_copy_kernel<false><<<(unsigned)(n < cap ? n : cap), 256, 0, (cudaStream_t)stream>>>(d_src, d_src_off, d_dst, d_dst_off, n);
+    HMSE_LAUNCH_CHECK(ctx);
+    return HMSE_OK;
+}
+
+int hmse_segment_gather(hmse_ctx* ctx, const uint64_t* d_src_addr, uint8_t* d_dst, const uint64_t* d_dst_off, uint64_t n,
+                        cudaStream_t stream) {
+    const uint64_t cap = (uint64_t)ctx->sm_count * 16;
+    KL(ctx);   // launched for n == 0 too, so that a caller's kernel count does not depend on n
+    segment_copy_kernel<true><<<(unsigned)(n == 0 ? 1 : n < cap ? n : cap), 256, 0, stream>>>(nullptr, d_src_addr, d_dst, d_dst_off, n);
     HMSE_LAUNCH_CHECK(ctx);
     return HMSE_OK;
 }

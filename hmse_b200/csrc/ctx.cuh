@@ -43,6 +43,7 @@ enum HmseSlot {
     SLOT_READ_PLAN,     // per-range lengths / first chunks / piece counts, need marks and their scans (hmse_read)
     SLOT_READ_WORK,     // need lists, per-stream statuses, piece offsets, gathered delta bytes
     SLOT_READ_DATA,     // the inflated stored chunks and applied deltas of one hmse_read batch
+    SLOT_COMPOSE,       // source table, first-reference keys, candidate lists, gathered digests, scans (hmse_compose)
     SLOT_COUNT
 };
 
@@ -52,7 +53,7 @@ constexpr int HMSE_MAX_WORLD = 32;          // ranks per communicator (the count
 constexpr size_t HMSE_MAILBOX_BYTES = 16384;
 enum HmseTimer {
     HT_SCAN = 0, HT_RESOLVE, HT_SHA, HT_DEDUP, HT_DEFLATE, HT_PACK, HT_MINHASH, HT_LSH, HT_INFLATE, HT_DELTA, HT_EXCHANGE,
-    HT_READ_PLAN, HT_READ_COPY, HT_COUNT
+    HT_READ_PLAN, HT_READ_COPY, HT_COMPOSE, HT_COUNT
 };
 
 struct hmse_ctx {
@@ -145,6 +146,17 @@ int hmse_inflate_ranges(hmse_ctx* ctx, const uint8_t* d_blob, const uint64_t* d_
                         const uint8_t* d_zdict, uint32_t dict_len, uint32_t dict_adler, uint8_t* d_out,
                         const uint64_t* d_out_offsets, uint32_t* d_status, cudaStream_t stream);
 uint32_t hmse_adler32_host(const uint8_t* d, size_t n);
+
+// hmse_dedup's table over n keys (stride bytes apart, the digest first): canon[i] = smallest j with key j == key i,
+// is_first[i] = (canon == i).  d_n (device, may be null) lowers n to a count only the device knows; the table is sized
+// for n.  Ends a streaming dedup session (SLOT_DEDUP_TABLE).  Asynchronous on `stream`.
+int hmse_dedup_table(hmse_ctx* ctx, const uint8_t* keys, uint64_t stride, uint64_t n, const uint64_t* d_n, int64_t* canon,
+                     uint8_t* is_first, uint64_t* canon_gid, cudaStream_t stream);
+
+// hmse_segment_copy with a source address per segment: d_dst[d_dst_off[i] : d_dst_off[i+1]) = the bytes at d_src_addr[i]
+// (4 readable bytes must follow every segment).  Asynchronous on `stream`.
+int hmse_segment_gather(hmse_ctx* ctx, const uint64_t* d_src_addr, uint8_t* d_dst, const uint64_t* d_dst_off, uint64_t n,
+                        cudaStream_t stream);
 
 // hmse_dedup_partition without the host round trip: d_counts[world] (device) receives the records per owner.
 int hmse_dedup_partition_dev(hmse_ctx* ctx, const uint8_t* d_digests, uint64_t n, uint64_t id_base, uint32_t world,

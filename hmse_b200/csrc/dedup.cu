@@ -40,11 +40,12 @@ __device__ __forceinline__ uint64_t slot_of(const Key& k, uint64_t mask) {
     return (h >> 20) & mask;
 }
 
-// Inserts keys i0 .. n-1 (earlier indices may already be in the table: streaming append).
+// Inserts keys i0 .. n-1 (earlier indices may already be in the table: streaming append); n_dev (device, may be null)
+// lowers n to a count only the device knows.
 __global__ void dedup_insert_kernel(const uint8_t* __restrict__ keys, uint64_t stride, uint64_t i0, uint64_t n,
-                                    uint32_t* __restrict__ table, uint64_t mask) {
+                                    const uint64_t* __restrict__ n_dev, uint32_t* __restrict__ table, uint64_t mask) {
     uint64_t i = i0 + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
+    if (i >= n || (n_dev && i >= *n_dev)) return;
     const Key me = load_key(keys, stride, i);
     uint64_t pos = slot_of(me, mask);
     for (;;) {
@@ -63,10 +64,10 @@ __global__ void dedup_insert_kernel(const uint8_t* __restrict__ keys, uint64_t s
 
 // Looks up keys i0 .. n-1; outputs are indexed from i0 (canon[i - i0] holds the absolute index).
 __global__ void dedup_lookup_kernel(const uint8_t* __restrict__ keys, uint64_t stride, uint64_t i0, uint64_t n,
-                                    const uint32_t* __restrict__ table, uint64_t mask, int64_t* __restrict__ canon,
-                                    uint8_t* __restrict__ is_first, uint64_t* __restrict__ canon_gid) {
+                                    const uint64_t* __restrict__ n_dev, const uint32_t* __restrict__ table, uint64_t mask,
+                                    int64_t* __restrict__ canon, uint8_t* __restrict__ is_first, uint64_t* __restrict__ canon_gid) {
     uint64_t i = i0 + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
+    if (i >= n || (n_dev && i >= *n_dev)) return;
     const Key me = load_key(keys, stride, i);
     uint64_t pos = slot_of(me, mask);
     for (;;) {
@@ -79,25 +80,6 @@ __global__ void dedup_lookup_kernel(const uint8_t* __restrict__ keys, uint64_t s
         }
         pos = (pos + 1) & mask;
     }
-}
-
-int run_table(hmse_ctx* ctx, const uint8_t* keys, uint64_t stride, uint64_t n, int64_t* canon, uint8_t* is_first,
-              uint64_t* canon_gid, cudaStream_t st) {
-    if (n >= 0x7FFFFFFFull) HMSE_FAIL(ctx, HMSE_E_INVAL, "dedup: more than 2^31-1 chunks per table");
-    uint64_t cap = 1024;
-    while (cap < 2 * n) cap <<= 1;
-    HMSE_SCRATCH(ctx, table, uint32_t*, SLOT_DEDUP_TABLE, cap * sizeof(uint32_t));
-    HMSE_CUDA(ctx, cudaMemsetAsync(table, 0xFF, cap * sizeof(uint32_t), st));
-    ctx->dedup_cap = 0;   // the one-shot table replaces a streaming one
-    const unsigned grid = (unsigned)div_up64(n, 256);
-    HT_BEGIN(ctx, HT_DEDUP, st);
-    KL(ctx);
-    dedup_insert_kernel<<<grid, 256, 0, st>>>(keys, stride, 0, n, table, cap - 1);
-    KL(ctx);
-    dedup_lookup_kernel<<<grid, 256, 0, st>>>(keys, stride, 0, n, table, cap - 1, canon, is_first, canon_gid);
-    HMSE_LAUNCH_CHECK(ctx);
-    HT_END(ctx, HT_DEDUP, st);
-    return HMSE_OK;
 }
 
 // ---- partition by owner ------------------------------------------------------------------
@@ -194,6 +176,25 @@ __global__ void select_scatter_kernel(const uint8_t* __restrict__ flags, const u
 
 }  // namespace
 
+int hmse_dedup_table(hmse_ctx* ctx, const uint8_t* keys, uint64_t stride, uint64_t n, const uint64_t* d_n, int64_t* canon,
+                     uint8_t* is_first, uint64_t* canon_gid, cudaStream_t st) {
+    if (n >= 0x7FFFFFFFull) HMSE_FAIL(ctx, HMSE_E_INVAL, "dedup: more than 2^31-1 chunks per table");
+    uint64_t cap = 1024;
+    while (cap < 2 * n) cap <<= 1;
+    HMSE_SCRATCH(ctx, table, uint32_t*, SLOT_DEDUP_TABLE, cap * sizeof(uint32_t));
+    HMSE_CUDA(ctx, cudaMemsetAsync(table, 0xFF, cap * sizeof(uint32_t), st));
+    ctx->dedup_cap = 0;   // the one-shot table replaces a streaming one
+    const unsigned grid = (unsigned)div_up64(n, 256);
+    HT_BEGIN(ctx, HT_DEDUP, st);
+    KL(ctx);
+    dedup_insert_kernel<<<grid, 256, 0, st>>>(keys, stride, 0, n, d_n, table, cap - 1);
+    KL(ctx);
+    dedup_lookup_kernel<<<grid, 256, 0, st>>>(keys, stride, 0, n, d_n, table, cap - 1, canon, is_first, canon_gid);
+    HMSE_LAUNCH_CHECK(ctx);
+    HT_END(ctx, HT_DEDUP, st);
+    return HMSE_OK;
+}
+
 HMSE_API int hmse_dedup_select(hmse_ctx* ctx, const uint8_t* d_is_first, uint64_t n, uint64_t* d_select, uint64_t cap,
                                uint64_t* m, void* stream) {
     if (!ctx) return HMSE_E_INVAL;
@@ -228,7 +229,7 @@ HMSE_API int hmse_dedup(hmse_ctx* ctx, const uint8_t* d_digests, uint64_t n, int
     if (n == 0) return HMSE_OK;
     if (!d_digests || !d_canon) HMSE_FAIL(ctx, HMSE_E_INVAL, "hmse_dedup: null pointer");
     if ((uintptr_t)d_digests & 7) HMSE_FAIL(ctx, HMSE_E_INVAL, "d_digests must be 8-byte aligned");
-    return run_table(ctx, d_digests, 32, n, d_canon, d_is_first, nullptr, (cudaStream_t)stream);
+    return hmse_dedup_table(ctx, d_digests, 32, n, nullptr, d_canon, d_is_first, nullptr, (cudaStream_t)stream);
 }
 
 HMSE_API int hmse_dedup_begin(hmse_ctx* ctx, uint64_t max_chunks, void* stream) {
@@ -260,9 +261,9 @@ HMSE_API int hmse_dedup_append(hmse_ctx* ctx, const uint8_t* d_digests_all, uint
     const uint64_t n = n_prev + n_new;
     HT_BEGIN(ctx, HT_DEDUP, st);
     KL(ctx);
-    dedup_insert_kernel<<<grid, 256, 0, st>>>(d_digests_all, 32, n_prev, n, table, ctx->dedup_cap - 1);
+    dedup_insert_kernel<<<grid, 256, 0, st>>>(d_digests_all, 32, n_prev, n, nullptr, table, ctx->dedup_cap - 1);
     KL(ctx);
-    dedup_lookup_kernel<<<grid, 256, 0, st>>>(d_digests_all, 32, n_prev, n, table, ctx->dedup_cap - 1, d_canon, d_is_first,
+    dedup_lookup_kernel<<<grid, 256, 0, st>>>(d_digests_all, 32, n_prev, n, nullptr, table, ctx->dedup_cap - 1, d_canon, d_is_first,
                                               nullptr);
     HMSE_LAUNCH_CHECK(ctx);
     HT_END(ctx, HT_DEDUP, st);
@@ -326,7 +327,7 @@ HMSE_API int hmse_dedup_records(hmse_ctx* ctx, const uint8_t* d_records, uint64_
     const unsigned grid = (unsigned)div_up64(m, 256);
     HT_BEGIN(ctx, HT_DEDUP, st);
     KL(ctx);
-    dedup_insert_kernel<<<grid, 256, 0, st>>>(d_records, 40, 0, m, table, cap - 1);
+    dedup_insert_kernel<<<grid, 256, 0, st>>>(d_records, 40, 0, m, nullptr, table, cap - 1);
     KL(ctx);
     min_gid_kernel<<<grid, 256, 0, st>>>(d_records, m, table, cap - 1, min_gid);
     KL(ctx);

@@ -37,7 +37,7 @@ extern "C" {
 #define HMSE_E_NOMEM (-4)    /* scratch allocation failed                      */
 #define HMSE_E_NCCL (-5)     /* NCCL is missing or a collective failed (text in hmse_last_error) */
 
-#define HMSE_ABI_VERSION 4
+#define HMSE_ABI_VERSION 5
 
 typedef struct hmse_ctx hmse_ctx;
 
@@ -80,6 +80,7 @@ int hmse_guard_check(hmse_ctx* ctx);
 #define HMSE_T_EXCHANGE 10 /* the NCCL part of the last hmse_chunk_sharded / hmse_dedup_global / hmse_lsh_exchange */
 #define HMSE_T_READ_PLAN 11 /* hmse_read steps 1-4: range checks, locate, pieces, need lists and their scans */
 #define HMSE_T_READ_COPY 12 /* hmse_read: the pieces copied into the output, statuses folded per range */
+#define HMSE_T_COMPOSE 13   /* hmse_compose: from the run checks to the last record written */
 int hmse_timing(hmse_ctx* ctx, int enable);
 int hmse_timing_ms(hmse_ctx* ctx, int id, float* ms);
 /* Kernels launched through this ctx since hmse_create. */
@@ -326,6 +327,45 @@ int hmse_read(hmse_ctx* ctx, const void* d_layout, uint64_t n, uint64_t m, uint6
               const uint8_t* d_delta_store, const uint8_t* d_zdict, uint32_t dict_len, const uint64_t* d_ranges,
               uint64_t R, uint8_t* d_out, uint64_t out_cap, uint64_t* d_out_off, uint64_t* total, uint32_t* d_status,
               uint64_t* n_bad, uint64_t* stats4, void* stream);
+
+/* ---- Compose: files of several opened archives merged or subset into one archive, on the device.  The output is the
+ *      archive one ingest of the selected files, in order, would have written when the sources keep no deltas: stored
+ *      chunks numbered by first reference, equal SHA-256 digests stored once across sources.  The library keeps no
+ *      per-archive state: every source comes with the layout hmse_read_open wrote for it. ------------------------------- */
+
+/* One source: the buffers an archive was opened on (hmse_read_open) and its dims.  d_delta_store may be null when
+ * n_delta == 0.  The stores need 4 readable bytes after their end. */
+typedef struct hmse_compose_src {
+    const void* d_layout;         /* written by hmse_read_open for these buffers and dims */
+    const uint8_t* d_index;       /* m 40-byte ChunkIndex entries (4-byte aligned) */
+    const uint8_t* d_pointers;    /* n 8-byte pointer records */
+    const uint8_t* d_store;       /* chunk store */
+    const uint8_t* d_delta_store; /* DeltaChunk records */
+    uint64_t n, m, n_delta;
+} hmse_compose_src;
+
+/* srcs[n_src] (host): the sources.  d_runs[n_runs][3] (device, u64) = {source, first chunk, chunk count}: the output
+ * stream is the runs' chunks back to back, n_out chunks in all (the counts must add up to n_out, n_out <= 2^32 - 2).
+ * Outputs (device, caller-owned): d_pointers[n_out] (8-byte aligned) = one pointer record per output chunk, raw length
+ * copied from the source pointer; d_index[index_cap] (4-byte aligned) = one ChunkIndex entry per kept stored chunk;
+ * d_store[store_cap] = their zlib streams, copied byte for byte; d_delta_store[delta_cap] = the DeltaChunk records.
+ * Rule: a stored chunk is kept when an output chunk references it, directly or as the base of a referenced DeltaChunk
+ * record; its key is the output position of its first reference (a record's reference to its base counts at the
+ * record's chunk).  Kept chunks with equal digests (their sources' index entries) are one chunk: the smaller key wins,
+ * references to the other are remapped.  Kept chunks are numbered and packed in key order; records, identified by
+ * (source, record), are written once each, numbered by first reference, their base remapped and the rest copied.
+ * DeltaChunk records are not deduplicated across sources (the container stores no digest for them).  Refcounts: one
+ * per pointer to the slot and one per written record on its base, saturating at 65535.
+ * out6 (host) = {n_out, stored chunks referenced (before the digest dedup), stored chunks kept, store bytes, records,
+ * delta-store bytes}.  HMSE_E_INVAL, before anything is written: a layout that does not match its source's dims,
+ * sources whose dictionaries differ in length or Adler-32, a run outside its source, counts that do not add up to
+ * n_out, or an output whose chunk store plus delta store reaches 2 TiB.  HMSE_E_CAPACITY: out6 holds the sizes
+ * needed and nothing is written.  hmse_compose uses hmse_dedup's table: it ends a streaming dedup session.  Two host
+ * round trips (the sizes, then an error word); the number of kernels does not depend on n_src, n_runs or the sizes.
+ * Synchronises `stream`. */
+int hmse_compose(hmse_ctx* ctx, const hmse_compose_src* srcs, uint32_t n_src, const uint64_t* d_runs, uint64_t n_runs,
+                 uint64_t n_out, uint8_t* d_pointers, uint8_t* d_index, uint64_t index_cap, uint8_t* d_store,
+                 uint64_t store_cap, uint8_t* d_delta_store, uint64_t delta_cap, uint64_t* out6, void* stream);
 
 /* ---- L4 similarity: replaces minhash_compute (README.md:2578-2597) and LSH banding
  *      (README.md:2231-2235). -------------------------------------------------------------- */
