@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libhmse_b200.so")
 
 HMSE_OK, HMSE_E_INVAL, HMSE_E_CAPACITY, HMSE_E_CUDA, HMSE_E_NOMEM, HMSE_E_NCCL = 0, -1, -2, -3, -4, -5
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 
 class HmseError(RuntimeError):
@@ -75,6 +75,9 @@ SIGNATURES = {
     "hmse_read_open": (_I, [_P, _P, _U64, _P, _U64, _U64, _P, _U64, _U64, _U64, _P, _U32, _P, _U64, _P]),
     "hmse_read": (_I, [_P, _P, _U64, _U64, _U64, _P, _P, _P, _U32, _P, _U64, _P, _U64, _P, _PU64, _P, _PU64, _PU64, _P]),
     "hmse_compose": (_I, [_P, C.POINTER(ComposeSrc), _U32, _P, _U64, _U64, _P, _P, _U64, _P, _U64, _P, _U64, _PU64, _P]),
+    "hmse_compress_known": (_I, [_P, C.POINTER(ComposeSrc), _P, _U64, _P, _P, _P, _U64, _P, _U32, _I, _P, _U64, _P, _PU64, _P,
+                                 _PU64, _P]),
+    "hmse_compress_known_pack": (_I, [_P, _P, _U64, _P, _U64, _P]),
     "hmse_minhash": (_I, [_P, _P, _U64, _P, _U64, _P, _U32, _P, _P]),
     "hmse_minhash_select": (_I, [_P, _P, _U64, _P, _P, _U64, _P, _U32, _P, _P]),
     "hmse_lsh_keys": (_I, [_P, _P, _U64, _U32, _U32, _P, _P]),

@@ -306,6 +306,30 @@ class Context:
         self.check(rc)
         return out[:total.value], offsets
 
+    def compress_known(self, src, d: torch.Tensor, cuts: torch.Tensor, digests: torch.Tensor, select: Optional[torch.Tensor],
+                       zdict: Optional[torch.Tensor], level: int = 6, start0: int = 0, out: Optional[torch.Tensor] = None):
+        """compress() against an opened archive (hmse_compress_known): `src` is the archive's _lib.ComposeSrc, `digests` the
+        SHA-256 of every chunk.  Streams the archive holds are copied from it, the others compressed; blob and offsets
+        equal compress()'s.  Returns (blob, offsets, known int64[m]: source slot copied or -1, stats4 = [streams copied,
+        bytes copied, streams compressed, raw bytes compressed])."""
+        m = cuts.numel() if select is None else select.numel()
+        offsets = self.empty(m + 1, torch.int64)
+        known = self.empty(max(m, 1), torch.int64)
+        total, st4 = C.c_uint64(0), (C.c_uint64 * 4)()
+        zp = zdict.data_ptr() if zdict is not None and zdict.numel() else None
+        zl = zdict.numel() if zdict is not None else 0
+        sp = select.data_ptr() if select is not None else None
+        cap = out.numel() if out is not None else 0
+        # as compress(): without a buffer the first call plans and sizes, the pack writes a blob of exactly that size
+        rc = self.lib.hmse_compress_known(self.h, C.byref(src), d.data_ptr(), start0, cuts.data_ptr(), digests.data_ptr(), sp, m,
+                                          zp, zl, level, out.data_ptr() if out is not None else None, cap, offsets.data_ptr(),
+                                          C.byref(total), known.data_ptr(), st4, self.stream)
+        if (out is None and rc == 0) or (rc == _lib.HMSE_E_CAPACITY and total.value > cap):
+            out = self.empty(max(1, total.value), torch.uint8)
+            rc = self.lib.hmse_compress_known_pack(self.h, offsets.data_ptr(), m, out.data_ptr(), out.numel(), self.stream)
+        self.check(rc)
+        return out[:total.value], offsets, known[:m], [int(x) for x in st4]
+
     def inflate(self, blob: torch.Tensor, offsets: torch.Tensor, out_offsets: torch.Tensor, zdict: Optional[torch.Tensor]):
         """(out uint8[out_offsets[-1]], status int32[m], n_bad): every stream inflated on the device."""
         m = offsets.numel() - 1

@@ -216,6 +216,14 @@ class Reader:
             start = np.concatenate([[0], np.cumsum(raw)])
             self.file_start = start[ar.file_chunk.astype(np.int64)]
 
+    def src(self) -> "_lib.ComposeSrc":
+        """The descriptor hmse_compose and hmse_compress_known take for this archive."""
+        d = _lib.ComposeSrc()
+        d.d_layout, d.d_index, d.d_pointers = self.layout.data_ptr(), self.index.data_ptr(), self.pointers.data_ptr()
+        d.d_store, d.d_delta_store = self.store.data_ptr(), self.dstore.data_ptr() if self.n_delta else None
+        d.n, d.m, d.n_delta = self.n, self.m, self.n_delta
+        return d
+
     def file_size(self, f) -> np.ndarray:
         return self.file_start[np.asarray(f) + 1] - self.file_start[np.asarray(f)]
 
@@ -367,11 +375,7 @@ def compose(parts, ctx: Optional[Context] = None, stats: Optional[dict] = None) 
     readers = [opened[id(parts[p][0])] for p in used]
     slot = {p: k for k, p in enumerate(used)}
     runs[:, 0] = [slot[int(p)] for p in runs[:, 0]]
-    descs = (_lib.ComposeSrc * len(readers))()
-    for d, rd in zip(descs, readers):
-        d.d_layout, d.d_index, d.d_pointers = rd.layout.data_ptr(), rd.index.data_ptr(), rd.pointers.data_ptr()
-        d.d_store, d.d_delta_store = rd.store.data_ptr(), rd.dstore.data_ptr() if rd.n_delta else None
-        d.n, d.m, d.n_delta = rd.n, rd.m, rd.n_delta
+    descs = (_lib.ComposeSrc * len(readers))(*[rd.src() for rd in readers])
     sb = sum(int(rd.ar.store.size) for rd in readers)
     dsb = sum(int(rd.ar.delta_store.size) for rd in readers if rd.n_delta)
     icap = min(n_out, sum(rd.m for rd in readers))

@@ -312,7 +312,7 @@ HMSE_API int hmse_compose(hmse_ctx* ctx, const hmse_compose_src* srcs, uint32_t 
     KL(ctx);
     compose_cand_kernel<<<grid_of(SM > SR ? SM : SR, ~0u), 256, 0, st>>>(W, SM, SR);
     HMSE_LAUNCH_CHECK(ctx);
-    if (int e = hmse_dedup_table(ctx, W.dig, 32, KU, W.uflag + n_out, W.canon, W.is_first, nullptr, st)) return e;
+    if (int e = hmse_dedup_table(ctx, W.dig, 32, KU, W.uflag + n_out, W.canon, W.is_first, nullptr, SLOT_DEDUP_TABLE, st)) return e;
     KL(ctx);
     compose_keep_kernel<<<grid_of(KU, ~0u), 256, 0, st>>>(W, KU);
     HMSE_LAUNCH_CHECK(ctx);

@@ -28,7 +28,7 @@ HMSE_API int hmse_create(int device, hmse_ctx** out) {
         delete c;
         return HMSE_E_CUDA;
     }
-    for (int i = 0; i < 2 * HT_COUNT; i++)
+    for (int i = 0; i < 2 * HT_EVENT_PAIRS; i++)
         if (cudaEventCreate(&c->ev[i]) != cudaSuccess) {
             delete c;
             return HMSE_E_CUDA;
@@ -48,7 +48,7 @@ HMSE_API void hmse_destroy(hmse_ctx* ctx) {
     hmse_comm_destroy(ctx);
     for (int i = 0; i < SLOT_COUNT; i++)
         if (ctx->slot[i]) cudaFree(ctx->slot_base[i]);
-    for (int i = 0; i < 2 * HT_COUNT; i++)
+    for (int i = 0; i < 2 * HT_EVENT_PAIRS; i++)
         if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     for (int i = 0; i < 2 * HMSE_PARSE_EVENTS; i++)
         if (ctx->pev[i]) cudaEventDestroy(ctx->pev[i]);
@@ -160,6 +160,12 @@ HMSE_API int hmse_timing_ms(hmse_ctx* ctx, int id, float* ms) {
     if (!ctx->ev_set[id]) HMSE_FAIL(ctx, HMSE_E_INVAL, "timer %d has not been recorded", id);
     HMSE_CUDA(ctx, cudaEventSynchronize(ctx->ev[2 * id + 1]));
     HMSE_CUDA(ctx, cudaEventElapsedTime(ms, ctx->ev[2 * id], ctx->ev[2 * id + 1]));
+    if (id == HT_KNOWN && ctx->ev_set[HT_KNOWN_MERGE]) {
+        float merge = 0.f;
+        HMSE_CUDA(ctx, cudaEventSynchronize(ctx->ev[2 * HT_KNOWN_MERGE + 1]));
+        HMSE_CUDA(ctx, cudaEventElapsedTime(&merge, ctx->ev[2 * HT_KNOWN_MERGE], ctx->ev[2 * HT_KNOWN_MERGE + 1]));
+        *ms += merge;
+    }
     return HMSE_OK;
 }
 

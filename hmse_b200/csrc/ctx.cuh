@@ -44,6 +44,8 @@ enum HmseSlot {
     SLOT_READ_WORK,     // need lists, per-stream statuses, piece offsets, gathered delta bytes
     SLOT_READ_DATA,     // the inflated stored chunks and applied deltas of one hmse_read batch
     SLOT_COMPOSE,       // source table, first-reference keys, candidate lists, gathered digests, scans (hmse_compose)
+    SLOT_KNOWN_TABLE,   // digest table of the known lookup (never the streaming dedup table)
+    SLOT_KNOWN,         // gathered digests, canon, plan and source addresses of hmse_compress_known
     SLOT_COUNT
 };
 
@@ -53,13 +55,17 @@ constexpr int HMSE_MAX_WORLD = 32;          // ranks per communicator (the count
 constexpr size_t HMSE_MAILBOX_BYTES = 16384;
 enum HmseTimer {
     HT_SCAN = 0, HT_RESOLVE, HT_SHA, HT_DEDUP, HT_DEFLATE, HT_PACK, HT_MINHASH, HT_LSH, HT_INFLATE, HT_DELTA, HT_EXCHANGE,
-    HT_READ_PLAN, HT_READ_COPY, HT_COMPOSE, HT_COUNT
+    HT_READ_PLAN, HT_READ_COPY, HT_COMPOSE, HT_KNOWN, HT_COUNT
 };
+// HMSE_T_KNOWN is two spans (the lookup before the compression of the novel chunks, the merge after it): this private
+// event pair holds the second, and hmse_timing_ms(HMSE_T_KNOWN) returns their sum
+constexpr int HT_KNOWN_MERGE = HT_COUNT;
+constexpr int HT_EVENT_PAIRS = HT_COUNT + 1;
 
 struct hmse_ctx {
     int device;
-    cudaEvent_t ev[2 * HT_COUNT];
-    uint8_t ev_set[HT_COUNT];
+    cudaEvent_t ev[2 * HT_EVENT_PAIRS];
+    uint8_t ev_set[HT_EVENT_PAIRS];
     int timing;
     uint64_t launches;  // kernels launched through this ctx
     char err[512];
@@ -87,6 +93,8 @@ struct hmse_ctx {
     void* dict_host;  // host copy + checksum of the indexed preset dictionary (deflate.cu)
     uint64_t pack_m, pack_total;  // streams / bytes staged by the last hmse_compress, still waiting in SLOT_DEFLATE_STAGE
     int pack_valid;               // (hmse_compress_pack copies them out without compressing again)
+    uint64_t known_m, known_total;  // streams / bytes planned by the last hmse_compress_known (source addresses in SLOT_KNOWN)
+    int known_valid;                // (hmse_compress_known_pack gathers them; any hmse_compress clears it)
     // multi-GPU (comm.cu)
     void* comm;       // ncclComm_t made by hmse_comm_init (null: callers pass their own)
     int comm_owned;
@@ -149,9 +157,14 @@ uint32_t hmse_adler32_host(const uint8_t* d, size_t n);
 
 // hmse_dedup's table over n keys (stride bytes apart, the digest first): canon[i] = smallest j with key j == key i,
 // is_first[i] = (canon == i).  d_n (device, may be null) lowers n to a count only the device knows; the table is sized
-// for n.  Ends a streaming dedup session (SLOT_DEDUP_TABLE).  Asynchronous on `stream`.
+// for n.  The table lives in scratch slot `slot`: SLOT_DEDUP_TABLE ends a streaming dedup session, any other slot
+// leaves it alone.  Asynchronous on `stream`.
 int hmse_dedup_table(hmse_ctx* ctx, const uint8_t* keys, uint64_t stride, uint64_t n, const uint64_t* d_n, int64_t* canon,
-                     uint8_t* is_first, uint64_t* canon_gid, cudaStream_t stream);
+                     uint8_t* is_first, uint64_t* canon_gid, int slot, cudaStream_t stream);
+
+// Where the streams staged by the last hmse_compress (m of them) sit: stream k starts at *stage + (*slot_off)[k] (device
+// addresses).  Valid until the next hmse_compress on ctx; HMSE_E_INVAL when nothing of m streams is staged.
+int hmse_compress_staged(hmse_ctx* ctx, uint64_t m, const uint8_t** stage, const uint64_t** slot_off);
 
 // hmse_segment_copy with a source address per segment: d_dst[d_dst_off[i] : d_dst_off[i+1]) = the bytes at d_src_addr[i]
 // (4 readable bytes must follow every segment).  Asynchronous on `stream`.

@@ -177,13 +177,13 @@ __global__ void select_scatter_kernel(const uint8_t* __restrict__ flags, const u
 }  // namespace
 
 int hmse_dedup_table(hmse_ctx* ctx, const uint8_t* keys, uint64_t stride, uint64_t n, const uint64_t* d_n, int64_t* canon,
-                     uint8_t* is_first, uint64_t* canon_gid, cudaStream_t st) {
+                     uint8_t* is_first, uint64_t* canon_gid, int slot, cudaStream_t st) {
     if (n >= 0x7FFFFFFFull) HMSE_FAIL(ctx, HMSE_E_INVAL, "dedup: more than 2^31-1 chunks per table");
     uint64_t cap = 1024;
     while (cap < 2 * n) cap <<= 1;
-    HMSE_SCRATCH(ctx, table, uint32_t*, SLOT_DEDUP_TABLE, cap * sizeof(uint32_t));
+    HMSE_SCRATCH(ctx, table, uint32_t*, slot, cap * sizeof(uint32_t));
     HMSE_CUDA(ctx, cudaMemsetAsync(table, 0xFF, cap * sizeof(uint32_t), st));
-    ctx->dedup_cap = 0;   // the one-shot table replaces a streaming one
+    if (slot == SLOT_DEDUP_TABLE) ctx->dedup_cap = 0;   // the one-shot table replaces a streaming one
     const unsigned grid = (unsigned)div_up64(n, 256);
     HT_BEGIN(ctx, HT_DEDUP, st);
     KL(ctx);
@@ -229,7 +229,7 @@ HMSE_API int hmse_dedup(hmse_ctx* ctx, const uint8_t* d_digests, uint64_t n, int
     if (n == 0) return HMSE_OK;
     if (!d_digests || !d_canon) HMSE_FAIL(ctx, HMSE_E_INVAL, "hmse_dedup: null pointer");
     if ((uintptr_t)d_digests & 7) HMSE_FAIL(ctx, HMSE_E_INVAL, "d_digests must be 8-byte aligned");
-    return hmse_dedup_table(ctx, d_digests, 32, n, nullptr, d_canon, d_is_first, nullptr, (cudaStream_t)stream);
+    return hmse_dedup_table(ctx, d_digests, 32, n, nullptr, d_canon, d_is_first, nullptr, SLOT_DEDUP_TABLE, (cudaStream_t)stream);
 }
 
 HMSE_API int hmse_dedup_begin(hmse_ctx* ctx, uint64_t max_chunks, void* stream) {

@@ -2013,6 +2013,7 @@ HMSE_API int hmse_compress(hmse_ctx* ctx, const uint8_t* d_data, uint64_t start0
     if (!total || !d_offsets) HMSE_FAIL(ctx, HMSE_E_INVAL, "hmse_compress: total/d_offsets is null");
     *total = 0;
     ctx->pack_valid = 0;
+    ctx->known_valid = 0;   // a plan of hmse_compress_known points into the stage this call overwrites
     if (dict_len > DICT_MAX) HMSE_FAIL(ctx, HMSE_E_INVAL, "dict_len must be <= 32768");
     if (dict_len && !d_zdict) HMSE_FAIL(ctx, HMSE_E_INVAL, "d_zdict is null");
     if (level != 0 && level != 6)
@@ -2290,6 +2291,13 @@ HMSE_API int hmse_compress(hmse_ctx* ctx, const uint8_t* d_data, uint64_t start0
         HMSE_FAIL(ctx, HMSE_E_CAPACITY, "d_out capacity %llu < %llu bytes", (unsigned long long)out_cap,
                   (unsigned long long)mail[0]);
     return hmse_compress_pack(ctx, d_offsets, m, d_out, out_cap, stream);
+}
+
+int hmse_compress_staged(hmse_ctx* ctx, uint64_t m, const uint8_t** stage, const uint64_t** slot_off) {
+    if (!ctx->pack_valid || m != ctx->pack_m) HMSE_FAIL(ctx, HMSE_E_INVAL, "no staged result of %llu streams", (unsigned long long)m);
+    *stage = (const uint8_t*)ctx->slot[SLOT_DEFLATE_STAGE] + 2;                     // pack_kernel's source of stream k
+    *slot_off = (const uint64_t*)ctx->slot[SLOT_DEFLATE_MISC] + m;   // [slot_size m][slot_off m] ...
+    return HMSE_OK;
 }
 
 HMSE_API int hmse_compress_pack(hmse_ctx* ctx, const uint64_t* d_offsets, uint64_t m, uint8_t* d_out, uint64_t out_cap,

@@ -29,6 +29,8 @@ class IngestResult:
     delta_blob: Optional[torch.Tensor] = None     # L4: uint8 packed deltas (chunk order)
     delta_offsets: Optional[torch.Tensor] = None  # L4: int64 [n + 1]
     file_chunk: Optional[torch.Tensor] = None     # files: int64 [F + 1] index of each file's first chunk (run(files=...))
+    known: Optional[torch.Tensor] = None          # known=: int64 [m] archive slot each stream was copied from, or -1
+    stats: Optional[dict] = None                  # known=: streams / bytes copied, streams / raw bytes compressed
 
     @property
     def n_chunks(self) -> int:
@@ -68,15 +70,49 @@ class Ingest:
         dblob, doffs = ctx.delta_encode(d, cuts, base, start0=start0)
         return base, dblob, doffs
 
+    def open_known(self, known, compress: bool):
+        """The archive of run(known=...), opened: a Reader is used as it is, an Archive is opened for the call; None when
+        the archive stores no chunk (nothing can be known).  Raises ValueError when its dictionary differs
+        from this ingest's or nothing is compressed."""
+        from .archive import Reader
+        if not compress:
+            raise ValueError("known= needs compress=True: it decides which streams are copied instead of compressed")
+        ar = known.ar if isinstance(known, Reader) else known
+        if bytes(ar.zdict) != bytes(self.zdict.cpu().numpy()):
+            raise ValueError("the archive's dictionary differs from the ingest's")
+        if ar.n_unique == 0:
+            return None
+        return known if isinstance(known, Reader) else Reader(known, self.ctx)
+
+    def compress_known(self, rd, d: torch.Tensor, cuts: torch.Tensor, digests: torch.Tensor, sel: torch.Tensor, start0: int = 0,
+                       out: Optional[torch.Tensor] = None, ctx: Optional[Context] = None):
+        """(blob, offsets, known, stats): the selected chunks compressed against the opened archive `rd`
+        (hmse_compress_known) - blob and offsets are what Context.compress returns."""
+        ctx = ctx or self.ctx
+        if rd is None:
+            blob, offs = ctx.compress(d, cuts, sel, self.zdict, self.level, start0=start0, out=out)
+            starts = torch.cat([torch.full((1,), start0, dtype=torch.int64, device=cuts.device), cuts[:-1]])
+            raw = int((cuts - starts)[sel].sum()) if sel.numel() else 0
+            kn = torch.full((sel.numel(),), -1, dtype=torch.int64, device=ctx.tdev)
+            return blob, offs, kn, dict(copied=0, copied_bytes=0, compressed=int(sel.numel()), compressed_raw_bytes=raw)
+        blob, offs, kn, st4 = ctx.compress_known(rd.src(), d, cuts, digests, sel, self.zdict, self.level, start0=start0, out=out)
+        return blob, offs, kn, dict(copied=st4[0], copied_bytes=st4[1], compressed=st4[2], compressed_raw_bytes=st4[3])
+
     def run(self, d: torch.Tensor, compress: bool = True, l4: Optional[SimConfig] = None, min_votes: int = 4,
-            files=None) -> IngestResult:
+            files=None, known=None) -> IngestResult:
         """l4: also run the similarity layer; first occurrences that keep a delta are not compressed (`select` lists
         the chunks of the chunk store only) and `base` / `delta_blob` / `delta_offsets` describe the deltas.
         files: the sizes of the files `d` holds back to back (a sequence or an integer tensor, zeros allowed).  Every
         file is then chunked on its own (hmse_chunk_files): no chunk spans two files, so equal files give equal chunks
         wherever they sit, and `file_chunk` records where each file's chunks begin.  Everything after chunking runs
-        unchanged over the one chunk list."""
+        unchanged over the one chunk list.
+        known: an archive (`Archive`, opened for the call, or an opened `Reader`) whose streams are reused: a stored chunk
+        whose digest and raw length the archive holds takes the archive's stream instead of being compressed
+        (hmse_compress_known).  Every field equals the run without `known` when the archive was written by this encoder at
+        the same level and dictionary; `known` (int64 [m]) names the archive slot each stream came from (-1: compressed)
+        and `stats` counts what was copied and compressed."""
         ctx = self.ctx
+        rd = self.open_known(known, compress) if known is not None else None
         d = ctx.stage(d)     # unchanged when it is aligned and has slack behind it; re-staged otherwise
         file_chunk = None
         if files is None:
@@ -91,12 +127,15 @@ class Ingest:
             base, dblob, doffs = self.similarity_delta(d, cuts, first, l4, min_votes)
             stored = first & (base < 0)
         sel = self.select_first(stored.view(torch.uint8))
-        if compress:
+        kn = stats = None
+        if known is not None:
+            blob, offs, kn, stats = self.compress_known(rd, d, cuts, digests, sel)
+        elif compress:
             blob, offs = ctx.compress(d, cuts, sel, self.zdict, self.level)
         else:
             blob, offs = ctx.empty(0, torch.uint8), ctx.empty(1, torch.int64).zero_()
         return IngestResult(cuts, digests, canon, first, sel, blob, offs, base=base, delta_blob=dblob, delta_offsets=doffs,
-                            file_chunk=file_chunk)
+                            file_chunk=file_chunk, known=kn, stats=stats)
 
 
 @dataclass
@@ -109,6 +148,8 @@ class HostIngestResult:
     blob: torch.Tensor        # uint8
     h2d_bytes: int = 0
     d2h_bytes: int = 0
+    known: Optional[torch.Tensor] = None   # run(known=...): int64 [m] archive slot each stream was copied from, or -1
+    stats: Optional[dict] = None           # run(known=...): summed over the pieces
 
     @property
     def n_chunks(self) -> int:
@@ -200,6 +241,7 @@ class IngestStream(Ingest):
                 "digests": torch.empty(cap_chunks * 32, dtype=torch.uint8, pin_memory=True),
                 "canon": torch.empty(cap_chunks, dtype=torch.int64, pin_memory=True),
                 "offsets": torch.empty(cap_chunks + 1, dtype=torch.int64, pin_memory=True),
+                "known": torch.empty(cap_chunks, dtype=torch.int64, pin_memory=True),
                 "blob": torch.empty(host_blob_cap, dtype=torch.uint8, pin_memory=True)}
         return cap_chunks, h
 
@@ -251,7 +293,10 @@ class IngestStream(Ingest):
             yield self.run(cur_h, host_blob_cap, compress)
             cur_h = nxt
 
-    def run(self, host_in: torch.Tensor, host_blob_cap: Optional[int] = None, compress: bool = True) -> HostIngestResult:
+    def run(self, host_in: torch.Tensor, host_blob_cap: Optional[int] = None, compress: bool = True,
+            known=None) -> HostIngestResult:
+        """known: as Ingest.run(known=...), piece by piece against the same archive (opened once per call); the result
+        equals the run without it, plus `known` and `stats`."""
         import queue
         import threading
         import time
@@ -259,6 +304,8 @@ class IngestStream(Ingest):
         if host_in.is_cuda or host_in.dtype != torch.uint8 or host_in.dim() != 1:
             raise TypeError("host_in must be a 1-D uint8 host tensor (pinned for asynchronous copies)")
         n = host_in.numel()
+        rd = self.open_known(known, compress) if known is not None else None
+        stats = dict(copied=0, copied_bytes=0, compressed=0, compressed_raw_bytes=0) if known is not None else None
         t_run = time.perf_counter()
 
         def mark(label):
@@ -383,8 +430,15 @@ class IngestStream(Ingest):
                         self._stage[j] = back.empty(want, torch.uint8)
                     if ev_out[j] is not None:
                         cur.wait_event(ev_out[j])      # the buffer's previous contents have left the device
-                    blob, offs = back.compress(rec["view"], rec["cuts"], rec["sel"], self.zdict, self.level,
-                                               start0=rec["start0"], out=self._stage[j])
+                    if known is not None:
+                        blob, offs, kn, st = self.compress_known(rd, rec["view"], rec["cuts"], rec["dg"], rec["sel"],
+                                                                 start0=rec["start0"], out=self._stage[j], ctx=back)
+                        rec["known"] = kn
+                        for key in stats:
+                            stats[key] += st[key]
+                    else:
+                        blob, offs = back.compress(rec["view"], rec["cuts"], rec["sel"], self.zdict, self.level,
+                                                   start0=rec["start0"], out=self._stage[j])
                     if blob.data_ptr() != self._stage[j].data_ptr():   # did not fit (poorly compressible): keep the larger one
                         self._stage[j] = blob
                     mk, bk = rec["sel"].numel(), blob.numel()
@@ -403,6 +457,8 @@ class IngestStream(Ingest):
                     if mk:
                         host["offsets"][1 + m_total:1 + m_total + mk].copy_(offs_abs, non_blocking=True)
                         host["blob"][blob_total:blob_total + bk].copy_(blob, non_blocking=True)
+                        if known is not None:
+                            host["known"][m_total:m_total + mk].copy_(rec["known"], non_blocking=True)
                         d2h += mk * 8 + bk
                         keep.append(offs_abs)
                         ev_out[k & 1] = torch.cuda.Event()
@@ -428,7 +484,8 @@ class IngestStream(Ingest):
         del keep
         return HostIngestResult(host["cuts"][:n_chunks], host["digests"][:n_chunks * 32].view(n_chunks, 32),
                                 host["canon"][:n_chunks], host["offsets"][:m_total + 1], host["blob"][:blob_total],
-                                h2d_bytes=n, d2h_bytes=d2h)
+                                h2d_bytes=n, d2h_bytes=d2h, known=host["known"][:m_total] if known is not None else None,
+                                stats=stats)
 
 
 class CFabric:

@@ -37,7 +37,7 @@ extern "C" {
 #define HMSE_E_NOMEM (-4)    /* scratch allocation failed                      */
 #define HMSE_E_NCCL (-5)     /* NCCL is missing or a collective failed (text in hmse_last_error) */
 
-#define HMSE_ABI_VERSION 5
+#define HMSE_ABI_VERSION 6
 
 typedef struct hmse_ctx hmse_ctx;
 
@@ -81,6 +81,8 @@ int hmse_guard_check(hmse_ctx* ctx);
 #define HMSE_T_READ_PLAN 11 /* hmse_read steps 1-4: range checks, locate, pieces, need lists and their scans */
 #define HMSE_T_READ_COPY 12 /* hmse_read: the pieces copied into the output, statuses folded per range */
 #define HMSE_T_COMPOSE 13   /* hmse_compose: from the run checks to the last record written */
+#define HMSE_T_KNOWN 14     /* hmse_compress_known: the lookup (steps 1-3) plus the stream lengths and offsets (step 5); the
+                               compression of the novel chunks is HMSE_T_DEFLATE, the gather into d_out HMSE_T_PACK */
 int hmse_timing(hmse_ctx* ctx, int enable);
 int hmse_timing_ms(hmse_ctx* ctx, int id, float* ms);
 /* Kernels launched through this ctx since hmse_create. */
@@ -366,6 +368,38 @@ typedef struct hmse_compose_src {
 int hmse_compose(hmse_ctx* ctx, const hmse_compose_src* srcs, uint32_t n_src, const uint64_t* d_runs, uint64_t n_runs,
                  uint64_t n_out, uint8_t* d_pointers, uint8_t* d_index, uint64_t index_cap, uint8_t* d_store,
                  uint64_t store_cap, uint8_t* d_delta_store, uint64_t delta_cap, uint64_t* out6, void* stream);
+
+/* ---- Compression against an opened archive: a new snapshot that is mostly in an archive already costs the DEFLATE of
+ *      what the archive lacks.  The library keeps no per-archive state: the archive comes as an hmse_compose_src
+ *      (the layout hmse_read_open wrote and its buffers), and its digest table is rebuilt on every call. ---------------- */
+
+/* hmse_compress with one more input, the archive `src`, and the SHA-256 of every chunk: d_digests[i][32] (device, 4-byte
+ * aligned) for chunk i.  For stream k (chunk i = d_select[k], or k when d_select is NULL):
+ *  - known: the smallest source slot whose index entry holds the digest of chunk i also holds a chunk of i's raw length
+ *    (the layout's ulen).  Stream k is then the source's stream of that slot, copied byte for byte from src->d_store.
+ *    DeltaChunk targets have no index entry and are never known.
+ *  - novel: every other stream is compressed exactly as hmse_compress compresses it.
+ * d_out, d_offsets[m+1], *total, the sizes-only call (d_out == NULL, out_cap == 0) and HMSE_E_CAPACITY follow
+ * hmse_compress, in selection order; in both cases the plan and the compressed novel streams stay in ctx until the next
+ * hmse_compress / hmse_compress_known, and hmse_compress_known_pack writes them - no chunk is compressed twice.
+ * The output equals hmse_compress's byte for byte whenever the source's streams were written by this encoder at the same
+ * level with the same dictionary (every archive that hmse_index_build or hmse_compose wrote from ingests at that level).
+ * The container does not record the level: streams of another level are copied as they are - valid streams of the same
+ * chunks that inflate correctly, but not the bytes hmse_compress would write.
+ * d_known[m] (device, may be NULL) = the source slot stream k was copied from, or -1 when it was compressed.
+ * stats4 (host, may be NULL) = {streams copied, bytes copied, streams compressed, raw bytes compressed}.
+ * HMSE_E_INVAL before anything is written: a layout that was not opened for src's n, m, n_delta, a dictionary whose length
+ * or Adler-32 differs from the source's, null or misaligned buffers (d_cuts, d_select, d_offsets, d_known 8-byte aligned;
+ * d_data as for hmse_compress).  The digest table has a scratch slot of its own: a streaming dedup session
+ * (hmse_dedup_begin / append) survives the call; its build is also recorded as HMSE_T_DEDUP.  One host round trip besides those of hmse_compress (the checks and
+ * counts); the kernels of the lookup and the merge do not depend on m or on the source.  Synchronises `stream`. */
+int hmse_compress_known(hmse_ctx* ctx, const hmse_compose_src* src, const uint8_t* d_data, uint64_t start0,
+                        const uint64_t* d_cuts, const uint8_t* d_digests, const uint64_t* d_select, uint64_t m,
+                        const uint8_t* d_zdict, uint32_t dict_len, int level, uint8_t* d_out, uint64_t out_cap,
+                        uint64_t* d_offsets, uint64_t* total, int64_t* d_known, uint64_t* stats4, void* stream);
+/* Writes the m streams planned by the last hmse_compress_known on ctx (same d_offsets) into d_out[0 : total). */
+int hmse_compress_known_pack(hmse_ctx* ctx, const uint64_t* d_offsets, uint64_t m, uint8_t* d_out, uint64_t out_cap,
+                             void* stream);
 
 /* ---- L4 similarity: replaces minhash_compute (README.md:2578-2597) and LSH banding
  *      (README.md:2231-2235). -------------------------------------------------------------- */
